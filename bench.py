@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    (CPU arm: the oracle port of the reference)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (also writes what the last timed step computed)
 
 A *step* is one pass of the hot path over one batch of synthetic windows: for every window,
 `n_starts` Nelder-Mead fits from random simplices (ab_neutral::run), best-of-starts, then `n_boot`
@@ -40,7 +41,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 SEED = 0xAB0B200
+DUMP_BYTES = 32_000_000  # --dump-outputs writes at most this many bytes of arrays
 GOLDEN_PED = os.path.join(ROOT, "tests", "golden", "pedigree.txt")
 METRIC = "ABneutral fits/sec (window x start x boot, f64)"
 
@@ -564,6 +567,23 @@ def make_inputs(ab, torch, W, first, NS, NB, shape, pool):
     return peds, probs, sx_t, idx_t
 
 
+def dump_outputs(out_dir, fit, rows, first, n_pairs):
+    """--dump-outputs: the arrays the timed path hands back (Batch.download_fit + download_boot), as float64 .npy files,
+    for a fixed seeded sample of windows that stays under DUMP_BYTES (every window when they fit).  The inputs depend on
+    the arguments only, so two builds of the project run with the same arguments can be compared file by file."""
+    W, NB = len(fit.best), rows.shape[1]
+    per_window = 8 * (len(fit.best.dtype.names) + 3 + 2 + 2 * n_pairs + 7 * NB)  # theta holds 4; + window, status
+    n = min(W, max(1, DUMP_BYTES // per_window))
+    win = np.sort(np.random.default_rng([SEED, W]).choice(W, n, replace=False))
+    out = {"window": first + win, "status": fit.status[win], "pred": fit.pred.reshape(W, n_pairs)[win],
+           "resid": fit.resid.reshape(W, n_pairs)[win], "boot_rows": rows[win]}
+    for f in fit.best.dtype.names:
+        out["best_" + f] = fit.best[f][win]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -579,7 +599,13 @@ def main():
     ap.add_argument("--no-experiments", action="store_true", help="skip the flagged experiments reported beside the contract line")
     ap.add_argument("--c5-sites", type=int, default=5_000_000)
     ap.add_argument("--no-full-window", action="store_true", help="reference arm: skip the one full 1000 + 100 window")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the fits and bootstrap rows of the last timed step to DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs the GPU arm on one GPU")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -679,6 +705,8 @@ def main():
     batch.run_boot()
     batch.sync()
     r = resident_run(batch, max(0, args.warmup - 1), args.steps, True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch.download_fit(), batch.download_boot()[0], first, N)
     clocks = r["clocks"]
     t_max = allmax(r["total_ms"])
     value = fits_per_step * args.steps / (t_max * 1e-3)
