@@ -137,6 +137,15 @@ def _load() -> C.CDLL:
         "abfit_plot_bootstrap": (C.c_int, [C.c_char_p, vp, vp, i32]),
         "abfit_window_counts": (C.c_int, [vp, vp]),
         "abfit_place_sites": (C.c_int, [vp, i32, vp, i64, vp, vp, vp, i64, vp, vp]),
+        "abfit_sim_tree_build": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(vp)]),
+        "abfit_sim_tree_from_arrays": (C.c_int, [i32, vp, vp, vp, C.POINTER(vp)]),
+        "abfit_sim_tree_info": (C.c_int, [vp, vp, vp, vp]),
+        "abfit_sim_tree_pairs": (C.c_int, [vp, vp, i32]),
+        "abfit_sim_tree_thresholds": (C.c_int, [vp, vp, vp]),
+        "abfit_sim_tree_free": (None, [vp]),
+        "abfit_sim_equilibrium": (C.c_int, [dbl, dbl, C.POINTER(dbl), C.POINTER(dbl)]),
+        "abfit_simulate": (C.c_int, [vp, vp, vp, i64, i64, vp, vp, vp]),
+        "abfit_simulate_device": (C.c_int, [vp, vp, vp, i64, i64, vp, vp, vp, C.POINTER(C.c_float)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
@@ -157,7 +166,9 @@ EXPORTED_SYMBOLS = (
     "abfit_batch_timing abfit_batch_flops_per_eval abfit_batch_fp64_instr_per_eval abfit_batch_uses_specialised_kernels abfit_jit_dump abfit_jit_last_error abfit_analyze abfit_window_counts abfit_place_sites "
     "abfit_parse_methylome_line abfit_parse_methylome_buffer abfit_parse_annotation_line abfit_pedigree_graph abfit_pedigree_build abfit_pedigree_info abfit_pedigree_rows abfit_pedigree_warnings "
     "abfit_pedigree_free abfit_format_f64 abfit_steady_state abfit_write_pedigree abfit_write_analysis abfit_format_analysis "
-    "abfit_write_npy_f64 abfit_write_metaprofile_results abfit_plot_metaplot abfit_plot_bootstrap"
+    "abfit_write_npy_f64 abfit_write_metaprofile_results abfit_plot_metaplot abfit_plot_bootstrap "
+    "abfit_sim_tree_build abfit_sim_tree_from_arrays abfit_sim_tree_info abfit_sim_tree_pairs abfit_sim_tree_thresholds "
+    "abfit_sim_tree_free abfit_sim_equilibrium abfit_simulate abfit_simulate_device"
 ).split()
 
 
@@ -524,6 +535,27 @@ class Context:
     def batch(self, probs: Sequence[Problem]) -> "Batch":
         return Batch(self, probs)
 
+    # -- simulated methylomes (ABneutral on a pedigree forest) -----------------------------------
+    def simulate(self, tree: "SimTree", alpha, beta, weight=None, p0uu=None, *, L: int, seed: int, missing_rate=0.0,
+                 first_site=0):
+        """sites [first_site, first_site + L) of every sampled node -> (status u8, posterior_max, meth_lvl), each
+        [n_samples, L], the inputs of dmatrix().  weight / p0uu default to the steady state (sim_equilibrium)."""
+        prm = _sim_params(alpha, beta, weight, p0uu, missing_rate, seed)
+        S = tree.n_samples
+        status, post, meth = np.empty((S, L), dtype=np.uint8), np.empty((S, L)), np.empty((S, L))
+        _check(_lib.abfit_simulate(self._h, tree._h, C.byref(prm), first_site, L, _ptr(status), _ptr(post), _ptr(meth)))
+        return status, post, meth
+
+    def simulate_device(self, tree: "SimTree", d_status: int, d_post: int, d_meth: int, alpha, beta, weight=None, p0uu=None,
+                        *, L: int, seed: int, missing_rate=0.0, first_site=0) -> float:
+        """simulate() into DEVICE arrays [n_samples][L] (raw pointers, e.g. torch tensors' data_ptr()) of this context's
+        device; returns when they are written.  -> device time of the simulation kernel (ms)"""
+        prm = _sim_params(alpha, beta, weight, p0uu, missing_rate, seed)
+        ms = C.c_float()
+        _check(_lib.abfit_simulate_device(self._h, tree._h, C.byref(prm), first_site, L, C.c_void_p(d_status),
+                                          C.c_void_p(d_post), C.c_void_p(d_meth), C.byref(ms)))
+        return ms.value
+
 
 class Batch:
     """Device-resident batch of windows (abfit_batch): upload / run / download are separate so
@@ -864,3 +896,146 @@ def pedigree_graph(nodelist: str, edgelist: str):
     _check(_lib.abfit_pedigree_graph(os.fsencode(nodelist), os.fsencode(edgelist), C.cast(C.byref(ns), C.c_void_p), files,
                                      1 << 20, C.cast(C.byref(npairs), C.c_void_p), _ptr(pairs), 1 << 16))
     return files.value.decode().split("\n")[:-1], pairs[:npairs.value].copy()
+
+
+# ---------------------------------------------------------------------------------------------
+# simulated methylomes: ABneutral run forward on a pedigree forest (include/abfit.h), and design studies
+# ---------------------------------------------------------------------------------------------
+class _SimParams(C.Structure):
+    _fields_ = [("alpha", C.c_double), ("beta", C.c_double), ("weight", C.c_double), ("p0uu", C.c_double),
+                ("missing_rate", C.c_double), ("seed", C.c_uint64)]
+
+
+def sim_equilibrium(alpha: float, beta: float):
+    """founders at the model's steady state -> (p0uu, weight): p0uu = p_uu_est(alpha, beta), weight = p_um / (p_um +
+    p_mm) (src/alphabeta.rs:62-79).  With p0uu = p_uu_est the fit's penalty target eqp = p0uu agrees with the truth."""
+    p, w = C.c_double(), C.c_double()
+    _check(_lib.abfit_sim_equilibrium(float(alpha), float(beta), C.byref(p), C.byref(w)))
+    return p.value, w.value
+
+
+def _sim_params(alpha, beta, weight, p0uu, missing_rate, seed) -> _SimParams:
+    if weight is None or p0uu is None:
+        p_eq, w_eq = sim_equilibrium(alpha, beta)
+        weight = w_eq if weight is None else weight
+        p0uu = p_eq if p0uu is None else p0uu
+    return _SimParams(float(alpha), float(beta), float(weight), float(p0uu), float(missing_rate), int(seed))
+
+
+class SimTree:
+    """A pedigree forest to simulate on (abfit_sim_tree).  SimTree(parent, generation, sampled): parent[v] = -1 for a
+    root; SimTree.from_files(nodelist, edgelist): the files of `alphabeta`.  Sampled nodes give the output rows in node
+    order; pairs() are their pedigree rows (i, j, t0, t1, t2), the order and values pedigree_graph() gives."""
+
+    def __init__(self, parent, generation, sampled, _handle=None):
+        h = _handle
+        if h is None:
+            par = np.ascontiguousarray(parent, dtype=np.int32)
+            gen = np.ascontiguousarray(generation, dtype=np.int32)
+            smp = np.ascontiguousarray(sampled, dtype=np.uint8)
+            if not (par.ndim == gen.ndim == smp.ndim == 1 and len(par) == len(gen) == len(smp)):
+                raise ValueError("parent, generation and sampled must be 1-D arrays of one length")
+            h = C.c_void_p()
+            _check(_lib.abfit_sim_tree_from_arrays(len(par), _ptr(par), _ptr(gen), _ptr(smp), C.byref(h)))
+        self._h = h
+        n, s, p = C.c_int32(), C.c_int32(), C.c_int32()
+        _check(_lib.abfit_sim_tree_info(h, C.byref(n), C.byref(s), C.byref(p)))
+        self.n_nodes, self.n_samples, self.n_pairs = n.value, s.value, p.value
+
+    @classmethod
+    def from_files(cls, nodelist: str, edgelist: str) -> "SimTree":
+        h = C.c_void_p()
+        _check(_lib.abfit_sim_tree_build(os.fsencode(nodelist), os.fsencode(edgelist), C.byref(h)))
+        return cls(None, None, None, _handle=h)
+
+    @classmethod
+    def lines(cls, n_lines: int, generations, sample_founder: bool = False) -> "SimTree":
+        """n_lines lines descending from one founder at generation 0, each sampled at the given generations (e.g. 8
+        lines x generations 1..20); unsampled generations in between are not nodes (an edge spans the gap)"""
+        gens = sorted(int(g) for g in generations)
+        parent, gen, smp = [-1], [0], [1 if sample_founder else 0]
+        for _ in range(n_lines):
+            prev = 0
+            for g in gens:
+                parent.append(prev)
+                gen.append(g)
+                smp.append(1)
+                prev = len(gen) - 1
+        return cls(parent, gen, smp)
+
+    def pairs(self) -> np.ndarray:
+        out = np.empty((max(self.n_pairs, 1), 5))
+        _check(_lib.abfit_sim_tree_pairs(self._h, _ptr(out), self.n_pairs))
+        return out[:self.n_pairs]
+
+    def thresholds(self, alpha, beta, weight=None, p0uu=None) -> np.ndarray:
+        """the per-node draw table [n_nodes, 6] (include/abfit.h, abfit_sim_tree_thresholds)"""
+        prm = _sim_params(alpha, beta, weight, p0uu, 0.0, 0)
+        out = np.empty((self.n_nodes, 6))
+        _check(_lib.abfit_sim_tree_thresholds(self._h, C.byref(prm), _ptr(out)))
+        return out
+
+    def pedigree(self, D) -> np.ndarray:
+        """[n_pairs, 4] rows (t0, t1, t2, D) from a dmatrix() D row (pair order (0,1),(0,2)..)"""
+        pr = self.pairs()
+        i, j = pr[:, 0].astype(np.int64), pr[:, 1].astype(np.int64)
+        S = self.n_samples
+        idx = i * S - i * (i + 1) // 2 + (j - i - 1)
+        return np.column_stack([pr[:, 2:5], np.asarray(D)[idx]])
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.abfit_sim_tree_free(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def design_study(ctxs, tree: SimTree, alpha, beta, weight=None, p0uu=None, *, L: int, n_replicates: int, n_starts=64,
+                 n_boot=100, seed=0, missing_rate=0.0, thr=0.99, use_true_p0uu=True, max_iters_fit=10000,
+                 max_iters_boot=1000):
+    """How tightly does a design determine alpha and beta?  Simulates n_replicates independent data sets of L sites on
+    `tree` and fits every one with alphabeta::run (multi-start fit + bootstrap):
+      1. one simulation of n_replicates * L sites into device memory of ctxs[0] (replicate r = sites [r L, (r+1) L));
+      2. one observed-divergence call with a window per replicate (dmatrix_device);
+      3. one problem per replicate from tree.pairs();
+      4. one batched fit (alphabeta_batch, or alphabeta_batch_multi over all contexts); all windows share one pedigree
+         time structure, so the batch runs on the specialised kernels when it is large enough.
+    use_true_p0uu: the problems' p0uu (and penalty target) is the simulated founder Pr(UU); otherwise the one the
+    pipeline estimates from meth_lvl, mean over samples of 1 - mean(meth_lvl) = P(UU) + P(UM) / 2 (the reference's
+    estimator, src/pedigree.rs:159-183), which is not P(UU).
+    Device memory: 17 bytes per sample-site of n_samples x n_replicates x L.
+    -> dict(theta [R,4] best alpha, beta, weight, intercept; status [R] fit status (0 = ok); analysis [R,32]
+    (abfit_analyze of the bootstrap); D [R,n_pairs]; p0uu [R] used; truth dict)"""
+    import torch
+
+    ctxs = list(ctxs) if isinstance(ctxs, (list, tuple)) else [ctxs]
+    prm = _sim_params(alpha, beta, weight, p0uu, missing_rate, seed)
+    R, S = int(n_replicates), tree.n_samples
+    if R <= 0 or L <= 0 or S < 2 or tree.n_pairs == 0:
+        raise ValueError("design_study needs n_replicates > 0, L > 0 and a tree with sampled pairs")
+    dev = torch.device("cuda", ctxs[0].device)
+    status = torch.empty((S, R * L), dtype=torch.uint8, device=dev)
+    post = torch.empty((S, R * L), dtype=torch.float64, device=dev)
+    meth = torch.empty((S, R * L), dtype=torch.float64, device=dev)
+    torch.cuda.synchronize(dev)
+    ctxs[0].simulate_device(tree, status.data_ptr(), post.data_ptr(), meth.data_ptr(), prm.alpha, prm.beta, prm.weight,
+                            prm.p0uu, L=R * L, seed=seed, missing_rate=missing_rate)
+    seg = np.arange(R + 1, dtype=np.int64) * L
+    dm = ctxs[0].dmatrix_device(status.data_ptr(), post.data_ptr(), meth.data_ptr(), S, R * L, thr=thr, seg_offsets=seg)
+    del status, post, meth
+    p0 = np.full(R, prm.p0uu) if use_true_p0uu else dm["p0uu"]
+    probs = [Problem(tree.pedigree(dm["D"][r]), float(p0[r]), float(p0[r]), 1.0) for r in range(R)]
+    sx = np.stack([gen_start_simplices(seed, r, n_starts, float(pb.pedigree[:, 3].max())) for r, pb in enumerate(probs)])
+    if len(ctxs) > 1:
+        res = alphabeta_batch_multi(ctxs, probs, sx, n_boot, seed, max_iters_fit=max_iters_fit, max_iters_boot=max_iters_boot)
+    else:
+        res = ctxs[0].alphabeta_batch(probs, sx, n_boot, seed, max_iters_fit=max_iters_fit, max_iters_boot=max_iters_boot)
+    return {"theta": res["best"]["theta"].copy(), "status": res["status"], "analysis": res["analysis"],
+            "D": np.stack([pb.pedigree[:, 3] for pb in probs]), "p0uu": p0,
+            "truth": {"alpha": prm.alpha, "beta": prm.beta, "weight": prm.weight, "p0uu": prm.p0uu,
+                      "missing_rate": prm.missing_rate, "seed": int(seed)}}

@@ -1511,6 +1511,24 @@ int abfit_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const doubl
                            cnt_out, p0uu_out, methsum_out, nvalid_out, kernel_ms, launches_out);
 }
 
+int abfit_simulate(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site, int64_t L,
+                   uint8_t *status, double *posterior_max, double *meth_lvl)
+{
+    if (!ctx) return ABFIT_ERR_ARG;
+    ABFIT_CUDA(cudaSetDevice(ctx->device));
+    return run_simulate(ctx->stream, ctx->prop.multiProcessorCount, tree, params, first_site, L, status, posterior_max, meth_lvl,
+                        false, nullptr);
+}
+
+int abfit_simulate_device(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
+                          int64_t L, uint8_t *d_status, double *d_posterior_max, double *d_meth_lvl, float *kernel_ms)
+{
+    if (!ctx) return ABFIT_ERR_ARG;
+    ABFIT_CUDA(cudaSetDevice(ctx->device));
+    return run_simulate(ctx->stream, ctx->prop.multiProcessorCount, tree, params, first_site, L, d_status, d_posterior_max,
+                        d_meth_lvl, true, kernel_ms);
+}
+
 // ---------------------------------------------------------------------------------------
 // bootstrap statistics (src/analysis.rs:50-98) — O(n_boot) host post-processing
 // ---------------------------------------------------------------------------------------

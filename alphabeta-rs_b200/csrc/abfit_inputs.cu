@@ -235,12 +235,7 @@ bool read_file(const char *path, std::string &out)
     return true;
 }
 
-struct Node {
-    size_t id;
-    std::string file, name;
-    uint32_t generation;
-    bool meth;
-};
+typedef abfit::ListNode Node;
 
 
 // nodelist + edgelist -> measured nodes and, for every pair of them connected in the pedigree graph, (i, j, t0, t1, t2)
@@ -253,44 +248,59 @@ struct PedGraph {
     std::vector<Pair> pairs;
 };
 
-int build_graph(const char *nodelist_path, const char *edgelist_path, PedGraph &g)
+}  // namespace
+
+// nodes: split on \n and \r, skip the header, id = index after the header (src/pedigree.rs:99-116); edges: the first
+// two fields of every line after the header (src/pedigree.rs:123-135), names not yet resolved
+int abfit::read_node_edge_lists(const char *nodelist_path, const char *edgelist_path, std::vector<ListNode> &nodes,
+                                std::vector<std::pair<std::string, std::string>> &edges)
 {
     std::string ntext, etext;
     if (!read_file(nodelist_path, ntext) || !read_file(edgelist_path, etext)) {
         abfit::set_error("cannot read the nodelist or the edgelist");
         return ABFIT_ERR_ARG;
     }
-    // nodes: split on \n and \r, skip the header, id = index after the header (src/pedigree.rs:99-116)
-    std::vector<Node> nodes;
     {
         const std::vector<std::string> lines = split_any(ntext, "\n\r");
         for (size_t li = 1; li < lines.size(); ++li) {
             const std::vector<std::string> e = split_any(lines[li], ",\t ");
             uint32_t gen;
             if (e.size() < 4 || !parse_u32(e[2], gen)) continue;
-            nodes.push_back(Node{li - 1, e[0], e[1], gen, e[3] == "Y"});
+            nodes.push_back(ListNode{li - 1, e[0], e[1], gen, e[3] == "Y"});
         }
     }
     if (nodes.empty()) {
         abfit::set_error("No nodes could be parsed from the nodelist");
         return ABFIT_ERR_ARG;
     }
-    struct Edge {
-        const Node *from, *to;
-    };
-    std::vector<Edge> edges;  // src/pedigree.rs:123-135
     {
         const std::vector<std::string> lines = split_any(etext, "\n\r");
         for (size_t li = 1; li < lines.size(); ++li) {
             const std::vector<std::string> e = split_any(lines[li], "\t ,");
-            if (e.size() < 2) continue;
-            const Node *a = nullptr, *b = nullptr;
-            for (auto &n : nodes)
-                if (!a && n.name == e[0]) a = &n;
-            for (auto &n : nodes)
-                if (!b && n.name == e[1]) b = &n;
-            if (a && b) edges.push_back(Edge{a, b});
+            if (e.size() >= 2) edges.emplace_back(e[0], e[1]);
         }
+    }
+    return 0;
+}
+
+namespace {
+
+int build_graph(const char *nodelist_path, const char *edgelist_path, PedGraph &g)
+{
+    std::vector<Node> nodes;
+    std::vector<std::pair<std::string, std::string>> names;
+    if (int rc = abfit::read_node_edge_lists(nodelist_path, edgelist_path, nodes, names)) return rc;
+    struct Edge {
+        const Node *from, *to;
+    };
+    std::vector<Edge> edges;  // src/pedigree.rs:123-135: edges naming an unknown node are dropped
+    for (auto &e : names) {
+        const Node *a = nullptr, *b = nullptr;
+        for (auto &n : nodes)
+            if (!a && n.name == e.first) a = &n;
+        for (auto &n : nodes)
+            if (!b && n.name == e.second) b = &n;
+        if (a && b) edges.push_back(Edge{a, b});
     }
     for (auto &n : nodes)
         if (n.meth) g.meas.push_back(n);

@@ -102,4 +102,22 @@ int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_pos
                    int *launches, float *ms /* optional [2]: pack pass, pair pass + finalisation */,
                    DivArena *arena = nullptr /* null: allocate and free inside the call */);
 
+// ---- pedigree lists (abfit_inputs.cu) ---------------------------------------------------
+struct ListNode {
+    size_t id;  // line index after the header
+    std::string file, name;
+    uint32_t generation;
+    bool meth;
+};
+// the parsed nodelist (lines that do not parse are skipped, as the reference skips them) and the (from, to) names of
+// every edgelist line; ABFIT_ERR_ARG when a file cannot be read or no node parses
+int read_node_edge_lists(const char *nodelist_path, const char *edgelist_path, std::vector<ListNode> &nodes,
+                         std::vector<std::pair<std::string, std::string>> &edges);
+
+// ---- simulation (abfit_simulate.cu) ------------------------------------------------------
+// sites [first_site, first_site + L) of every sampled node of `tree` into status / posterior_max / meth_lvl, which are
+// device arrays (device_out) or host arrays (staged through device buffers); kernel_ms optional
+int run_simulate(cudaStream_t st, int n_sms, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
+                 int64_t L, uint8_t *status, double *posterior_max, double *meth_lvl, bool device_out, float *kernel_ms);
+
 }  // namespace abfit

@@ -373,6 +373,51 @@ int abfit_write_metaprofile_results(const char *path, const char *run_name, int3
                                     const int32_t *region, const abfit_fit *best, const double *analysis,
                                     const double *obs_steady_state);
 
+/* ---- simulated methylomes under ABneutral (data with known epimutation rates) --------------------------
+ * A pedigree forest: every node has at most one parent, generations do not decrease from parent to child and lie in
+ * 0..127 (the `as i8` time cast of src/divergence.rs:52).  A root at generation g draws its state (UU, UM, MM) from
+ * sv0.G^g with sv0 = [p0uu, w(1-p0uu), (1-w)(1-p0uu)] (divergence()'s sv0 with p0mm = 1 - p0uu, p0um = 0,
+ * src/ab_neutral.rs:23-24); a child draws from row state(parent) of G^(gen(child) - gen(parent)), G = genmatrix(alpha,
+ * beta), powers by matrix_power's chain under the arithmetic contract above.  Every sampled node gives one output row:
+ * status 0/1/2 (U/I/M), meth_lvl = status / 2, posterior_max = 1, or 0.5 with probability missing_rate (independent per
+ * sample and site).  Measurement error (the fit's intercept) is not simulated.
+ * Randomness is counter-based: every draw is keyed by (seed, node index, global site index), so a site range gives the
+ * same bits whether it is simulated in one call, in several calls (first_site) or on several devices. */
+typedef struct abfit_sim_tree abfit_sim_tree;
+typedef struct {
+    double alpha, beta;  /* per-generation gain / loss rates, [0, 1] */
+    double weight, p0uu; /* founder distribution (see above), [0, 1]; abfit_sim_equilibrium gives the steady state */
+    double missing_rate; /* [0, 1] */
+    uint64_t seed;
+} abfit_sim_params;
+/* nodelist + edgelist (the files abfit_pedigree_build reads; an edge's `from` is the parent).  Refused with
+ * ABFIT_ERR_ARG: a node with two parents, a cycle, gen(from) > gen(to), a generation above 127, an edge naming an
+ * unknown node.  Sampled nodes (meth == Y) give the output rows, in nodelist order. */
+int abfit_sim_tree_build(const char *nodelist_path, const char *edgelist_path, abfit_sim_tree **out);
+/* the same from arrays: parent [n_nodes] (-1 = root), generation [n_nodes], sampled [n_nodes] (0 / 1) */
+int abfit_sim_tree_from_arrays(int32_t n_nodes, const int32_t *parent, const int32_t *generation, const uint8_t *sampled,
+                               abfit_sim_tree **out);
+int abfit_sim_tree_info(const abfit_sim_tree *t, int32_t *n_nodes, int32_t *n_samples, int32_t *n_pairs);
+/* pedigree rows (i, j, t0, t1, t2) of the sampled nodes, in the order and with the values abfit_pedigree_graph gives
+ * for the same files: the D column of pair (i, j) is entry (i, j) of abfit_divergence on the simulated rows */
+int abfit_sim_tree_pairs(const abfit_sim_tree *t, double *pairs_out /*[n_pairs][5]*/, int32_t pairs_cap);
+/* the per-node draw table [n_nodes][6]: for parent state k the pair (c0, c1) = (r0, r0 + r1) of row k of G^delta; a
+ * root's pair (of sv0.G^g) is stored three times.  A draw u in [0, 1) gives u < c0 ? 0 : u < c1 ? 1 : 2. */
+int abfit_sim_tree_thresholds(const abfit_sim_tree *t, const abfit_sim_params *params, double *out);
+void abfit_sim_tree_free(abfit_sim_tree *t);
+/* the founders at the model's steady state: p0uu = p_uu_est(alpha, beta), weight = p_um / (p_um + p_mm)
+ * (src/alphabeta.rs:62-79, src/structs.rs:146-159) */
+int abfit_sim_equilibrium(double alpha, double beta, double *p0uu_out, double *weight_out);
+/* sites [first_site, first_site + L) of every sampled node into host arrays status [S][L] u8, posterior_max [S][L],
+ * meth_lvl [S][L] (the layout abfit_divergence reads) */
+int abfit_simulate(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site, int64_t L,
+                   uint8_t *status, double *posterior_max, double *meth_lvl);
+/* the same into device arrays (e.g. the inputs of abfit_divergence_device: 17 bytes per sample-site never cross
+ * PCIe); runs on the context stream and returns when the arrays are written.  kernel_ms: device time of the
+ * simulation kernel (may be NULL). */
+int abfit_simulate_device(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
+                          int64_t L, uint8_t *d_status, double *d_posterior_max, double *d_meth_lvl, float *kernel_ms);
+
 /* ---- the reference's pictures (host; src/plot.rs) ------------------------------------
  * 1280 x 960 PNG files with the reference's series, colours, axis ranges and captions (not its pixels: own
  * rasteriser and bitmap font, see csrc/abfit_plot.cu).
