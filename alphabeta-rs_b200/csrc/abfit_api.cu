@@ -1330,11 +1330,12 @@ int abfit_model_divergence(abfit_ctx *ctx, const abfit_problem *prob, const doub
 }
 
 // pitch: row stride (in sites) of the three HOST arrays when they are column slices of wider matrices (0: L)
+// long_windows: run_divergence's argument (a shard of abfit_divergence_multi passes its whole call's div_long_windows)
 static int divergence_impl(abfit_ctx *ctx, bool device_inputs, const uint8_t *status, const double *posterior_max,
                            const double *meth_lvl, int32_t S, int64_t L, const int64_t *seg_offsets, int32_t W,
                            double thr, double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out,
                            double *methsum_out, int64_t *nvalid_out, float *ms_out, int32_t *launches_out,
-                           int64_t pitch = 0)
+                           int64_t pitch = 0, int long_windows = -1)
 {
     if (!ctx || !status || !posterior_max || !meth_lvl || S <= 0 || L < 0 || S > 65535) return ABFIT_ERR_ARG;
     int64_t whole[2] = {0, L};
@@ -1383,7 +1384,8 @@ static int divergence_impl(abfit_ctx *ctx, bool device_inputs, const uint8_t *st
     int launches = 0;
     if (int rc = run_divergence(st, device_inputs ? status : d_status.p, device_inputs ? posterior_max : d_post.p,
                                 device_inputs ? meth_lvl : d_meth.p, S, L, seg_offsets, W, thr, d_D.p, d_diff.p,
-                                d_cnt.p, d_methsum.p, d_nvalid.p, d_p0uu.p, &launches, ms_out, &ctx->div_arena))
+                                d_cnt.p, d_methsum.p, d_nvalid.p, d_p0uu.p, &launches, ms_out, &ctx->div_arena,
+                                long_windows))
         return rc;
     if (launches_out) *launches_out = launches;
     if (D_out && P) ABFIT_CUDA(cudaMemcpyAsync(D_out, d_D.p, (size_t)W * P * 8, cudaMemcpyDeviceToHost, st));
@@ -1414,9 +1416,17 @@ int abfit_divergence_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const uint8_t 
     for (int r = 0; r < n_ctx; ++r)
         if (!ctxs[r]) return ABFIT_ERR_ARG;
     const size_t P = (size_t)S * (S - 1) / 2;
-    if (seg_offsets && W > 1) {
-        // windows are independent: every device takes a contiguous block of windows (and the site range they cover);
-        // results are per window, so this is the single-device result bit for bit
+    if (seg_offsets) {
+        // windows are independent: every device takes a contiguous block of windows (and the site range they cover).
+        // Results are per window, and every shard sums meth_lvl in the tree one device would choose for the whole
+        // window list (div_long_windows), so this is the single-device result bit for bit.  One window stays on one
+        // device: only seg_offsets == NULL shards the site axis.
+        if (W <= 0) return ABFIT_ERR_ARG;
+        if (seg_offsets[0] < 0 || seg_offsets[W] > L) {
+            set_error("seg_offsets outside [0, L]");
+            return ABFIT_ERR_ARG;
+        }
+        const int long_windows = div_long_windows(seg_offsets, W) ? 1 : 0;
         const int world = std::min<int>(n_ctx, W);
         std::vector<int> rcs(world, 0);
         std::vector<std::string> errs(world);
@@ -1430,7 +1440,7 @@ int abfit_divergence_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const uint8_t 
                                      thr, D_out ? D_out + (size_t)w0 * P : nullptr, diff_out ? diff_out + (size_t)w0 * P : nullptr,
                                      cnt_out ? cnt_out + (size_t)w0 * P : nullptr, p0uu_out ? p0uu_out + w0 : nullptr,
                                      methsum_out ? methsum_out + (size_t)w0 * S : nullptr,
-                                     nvalid_out ? nvalid_out + (size_t)w0 * S : nullptr, nullptr, nullptr, L);
+                                     nvalid_out ? nvalid_out + (size_t)w0 * S : nullptr, nullptr, nullptr, L, long_windows);
             if (rcs[r]) errs[r] = g_last_error;
         };
         std::vector<std::thread> th;
@@ -1444,15 +1454,11 @@ int abfit_divergence_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const uint8_t 
             }
         return 0;
     }
-    // one window = all sites (whole methylomes, BASELINE configs[4]): the SITE axis is sharded in 64-site words; the
-    // integer partial sums add up exactly, so D = diff / (2 cnt) (src/pedigree.rs:257) does not depend on the number
-    // of devices; the per-sample methylation sums are added in device order (p0uu within 1e-12 of one device)
-    const int64_t a0 = seg_offsets ? seg_offsets[0] : 0, b0 = seg_offsets ? seg_offsets[1] : L;
-    if (a0 < 0 || b0 > L || b0 < a0) {
-        set_error("seg_offsets outside [0, L]");
-        return ABFIT_ERR_ARG;
-    }
-    const int64_t words = (b0 - a0 + 63) / 64;
+    // no seg_offsets: one window = all sites (whole methylomes, BASELINE configs[4]): the SITE axis is sharded in
+    // 64-site words; the integer partial sums add up exactly, so D = diff / (2 cnt) (src/pedigree.rs:257) does not
+    // depend on the number of devices; the per-sample methylation sums are added in device order (p0uu within 1e-12 of
+    // one device)
+    const int64_t words = (L + 63) / 64;
     const int world = (int)std::max<int64_t>(1, std::min<int64_t>(n_ctx, words));
     std::vector<std::vector<uint64_t>> pd(world, std::vector<uint64_t>(P)), pc(world, std::vector<uint64_t>(P));
     std::vector<std::vector<double>> pm(world, std::vector<double>(S));
@@ -1462,7 +1468,7 @@ int abfit_divergence_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const uint8_t 
     auto work = [&](int r) {
         int64_t w0, wc;
         shard_range(words, r, world, w0, wc);
-        const int64_t a = std::min(a0 + w0 * 64, b0), b = std::min(a0 + (w0 + wc) * 64, b0);
+        const int64_t a = std::min(w0 * 64, L), b = std::min((w0 + wc) * 64, L);
         rcs[r] = divergence_impl(ctxs[r], false, status + a, posterior_max + a, meth_lvl + a, S, b - a, nullptr, 1, thr, nullptr,
                                  pd[r].data(), pc[r].data(), nullptr, pm[r].data(), pn[r].data(), nullptr, nullptr, L);
         if (rcs[r]) errs[r] = g_last_error;

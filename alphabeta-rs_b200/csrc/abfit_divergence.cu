@@ -794,11 +794,19 @@ static size_t fused_smem(int S, int pack_warps, int ring)
     return (size_t)pack_warps * ring * FUSED_SLOT + (size_t)2 * 3 * FUSED_GW * Sp * 8 + (size_t)(4 + pack_warps * ring) * 8;
 }
 
+bool div_long_windows(const int64_t *h_seg, int W)
+{
+    // (a few long windows — chromosomes — run the kernel once each)
+    bool all_long = W >= 1 && W <= 64;
+    for (int w = 0; w < W && all_long; ++w) all_long = h_seg[w + 1] - h_seg[w] > EXACT_MAX;
+    return all_long;
+}
+
 // -------------------------------------------------------------------------------------
 int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_post, const double *d_meth, int S,
                    int64_t L, const int64_t *h_seg, int W, double thr, double *d_D, unsigned long long *d_diff,
                    unsigned long long *d_cnt, double *d_methsum, long long *d_nvalid, double *d_p0uu,
-                   int *launches, float *ms, DivArena *arena)
+                   int *launches, float *ms, DivArena *arena, int long_windows)
 {
     // host-side segmentation tables
     std::vector<SuperBlock> sbs;
@@ -841,9 +849,7 @@ int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_pos
         int pack_warps = 8, ring = 2;
         if (const char *e = getenv("ABFIT_DEV_DIV_FUSED_SHAPE")) sscanf(e, "%dx%d", &pack_warps, &ring);
         const int nb_f = (S + 3) / 4, n_tiles_f = nb_f * (nb_f + 1) / 2;
-        // (a few long windows — chromosomes — run the kernel once each)
-        bool all_long = W >= 1 && W <= 64;
-        for (int w = 0; w < W && all_long; ++w) all_long = h_seg[w + 1] - h_seg[w] > EXACT_MAX;
+        const bool all_long = long_windows >= 0 ? long_windows != 0 : div_long_windows(h_seg, W);
         const bool can = all_long && P > 0 && n_tiles_f <= 2 * PAIR_THREADS_MAX && fused_smem(S, pack_warps, ring) <= (size_t)smem_optin;
         bool fused = can;
         if (const char *e = getenv("ABFIT_DEV_DIV_FUSED")) fused = atoi(e) != 0 && can;

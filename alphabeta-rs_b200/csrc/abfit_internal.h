@@ -100,7 +100,12 @@ int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_pos
                    int64_t L, const int64_t *h_seg, int W, double thr, double *d_D, unsigned long long *d_diff,
                    unsigned long long *d_cnt, double *d_methsum, long long *d_nvalid, double *d_p0uu,
                    int *launches, float *ms /* optional [2]: pack pass, pair pass + finalisation */,
-                   DivArena *arena = nullptr /* null: allocate and free inside the call */);
+                   DivArena *arena = nullptr /* null: allocate and free inside the call */,
+                   int long_windows = -1 /* 0 / 1: what div_long_windows said of the whole call, -1: of h_seg */);
+// The window list qualifies for the fused kernel: 1 to 64 windows, each of more than 65 536 sites.  The fused and the
+// two-pass path sum meth_lvl in different trees, so a call that is split over devices decides this once, for all of
+// its windows, and passes the answer to every shard: each window then gets the bits one device gives it.
+bool div_long_windows(const int64_t *h_seg, int W);
 
 // ---- pedigree lists (abfit_inputs.cu) ---------------------------------------------------
 struct ListNode {

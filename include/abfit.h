@@ -202,10 +202,12 @@ int abfit_alphabeta_batch_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const abf
 
 /* Observed pairwise divergence + p0uu.  Replaces `DMatrix::from` (src/pedigree.rs:213-262)
  * and the per-sample statistics of `Pedigree::build` (src/pedigree.rs:159-183).
- *  status        [S][L] u8: 0 = U, 1 = I, 2 = M (src/methylation_site.rs:130-136)
+ *  status        [S][L] u8: 0 = U, 1 = I, 2 = M (src/methylation_site.rs:130-136); other values are not
+ *                checked and count as 2
  *  posterior_max [S][L], meth_lvl [S][L] (rc.meth.lvl)
  *  seg_offsets   [W+1] site ranges of W windows over the L axis, or NULL (one window = all sites)
- *  thr           posterior_max_filter (0.99)
+ *  thr           posterior_max_filter (0.99).  A site is valid where posterior_max >= thr: a NaN posterior, or
+ *                thr = NaN, makes it invalid (src/pedigree.rs:249-251); meth_lvl of an invalid site is never read
  *  D_out    [W][S(S-1)/2]  diff/(2*cnt) in pair order (0,1),(0,2)...(S-2,S-1); 0/0 = NaN
  *  diff_out, cnt_out [W][S(S-1)/2] exact integer sums (may be NULL)
  *  p0uu_out [W] = mean_s(1 - methsum/nvalid) (may be NULL)
@@ -218,17 +220,21 @@ int abfit_divergence(abfit_ctx *ctx, const uint8_t *status, const double *poster
                      uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out, double *methsum_out,
                      int64_t *nvalid_out);
 
-/* abfit_divergence over several GPUs (one context per device).  W > 1: the WINDOWS are sharded (results are per
- * window: bit-identical to one device).  One window = whole methylomes (src/pedigree.rs:213-262 at 200 x 5 M sites):
- * the SITE axis is sharded; the exact integer sums of every shard are added on the host, so D is bit-identical for any
- * number of devices, and p0uu agrees within 1e-12 (per-sample sums added in device order). */
+/* abfit_divergence over several GPUs (one context per device).  With seg_offsets the WINDOWS are sharded: every
+ * shard sums meth_lvl in the tree one device picks for the whole window list, so all outputs are bit-identical to
+ * abfit_divergence on one device, for any W (W = 1 runs on the first context).  seg_offsets = NULL (whole
+ * methylomes, src/pedigree.rs:213-262 at 200 x 5 M sites): the SITE axis is sharded; the exact integer sums of every
+ * shard are added on the host, so D is bit-identical for any number of devices, and p0uu agrees within 1e-12
+ * (per-sample sums added in device order). */
 int abfit_divergence_multi(abfit_ctx *const *ctxs, int32_t n_ctx, const uint8_t *status, const double *posterior_max,
                            const double *meth_lvl, int32_t S, int64_t L, const int64_t *seg_offsets, int32_t W, double thr,
                            double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out, double *methsum_out,
                            int64_t *nvalid_out);
 
 /* The same with the three input arrays already in device memory (site tables that stay resident between
- * calls; bench: HBM roofline of the packing pass).  seg_offsets and all outputs are host memory.
+ * calls; bench: HBM roofline of the packing pass).  seg_offsets and all outputs are host memory.  The call runs on
+ * the context's own non-blocking stream, which does not wait for work on other streams: the inputs must be complete
+ * (e.g. the stream that wrote them synchronised) before the call.
  * kernel_ms[0] = device time of the packing pass (streams 17 B per sample-site), kernel_ms[1] = all-pairs
  * popcounts + finalisation; launches_out = kernels launched.  Both may be NULL. */
 int abfit_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const double *d_posterior_max,

@@ -660,7 +660,9 @@ void abref_dmatrix(const uint8_t *status, const double *post, int S, int64_t L, 
             const uint8_t *si = status + (size_t)i * L, *sj = status + (size_t)j * L;
             const double *pi = post + (size_t)i * L, *pj = post + (size_t)j * L;
             for (int64_t k = 0; k < L; ++k) {
-                if (pi[k] < thr || pj[k] < thr) continue;
+                /* src/pedigree.rs:249-251 keeps a site when post_i >= thr && post_j >= thr: a NaN posterior (or
+                 * thr = NaN) fails the test, as in abref_p0uu */
+                if (!(pi[k] >= thr && pj[k] >= thr)) continue;
                 int a = si[k], b = sj[k];
                 div += (uint64_t)(a > b ? a - b : b - a);
                 cnt += 1;

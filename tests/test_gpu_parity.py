@@ -1212,6 +1212,7 @@ def test_c5_full_size_divergence_properties(ab, ctx, oracle):
         u = torch.rand(L, device=dev, generator=g, dtype=torch.float64)
         post[s] = torch.where(torch.rand(L, device=dev, generator=g) < 0.9, torch.full_like(u, 0.9999), u * 0.49 + 0.5)
         meth[s] = torch.rand(L, device=dev, generator=g, dtype=torch.float64)
+    torch.cuda.synchronize()  # the library's stream does not wait for torch's: the inputs must be complete first
     run = lambda seg=None: ctx.dmatrix_device(status.data_ptr(), post.data_ptr(), meth.data_ptr(), S, L, 0.99, seg_offsets=seg)
     whole = run()
     assert whole["launches"] <= 4  # the fused kernel

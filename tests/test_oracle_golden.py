@@ -176,12 +176,18 @@ def test_sanity_anchor_small_pedigree(ab, oracle):
 
 
 def test_dmatrix_edge_cases(oracle):
-    """empty overlap -> NaN (0/0), all-equal -> 0, max distance -> 1"""
-    st = np.array([[0, 1, 2, 2], [2, 1, 0, 2], [0, 0, 0, 0]], dtype=np.uint8)
-    po = np.array([[1, 1, 1, 0.5], [1, 1, 1, 1], [0.1, 0.1, 0.1, 0.1]])
+    """empty overlap -> NaN (0/0), all-equal -> 0, max distance -> 1; a site is kept when post_i >= thr && post_j >= thr
+    (src/pedigree.rs:249-251): a NaN posterior drops it, as it does from p0uu, and thr = NaN keeps none"""
+    st = np.array([[0, 1, 2, 2, 0], [2, 1, 0, 2, 2], [0, 0, 0, 0, 0]], dtype=np.uint8)
+    po = np.array([[1, 1, 1, 0.5, np.nan], [1, 1, 1, 1, 1], [0.1, 0.1, 0.1, 0.1, 0.1]])
     D, diff, cnt = oracle.dmatrix(st, po, 0.99)
     assert diff[0] == 4 and cnt[0] == 3 and D[0] == 4 / 6
     assert np.isnan(D[1]) and np.isnan(D[2]) and cnt[1] == 0
+    _, _, nv = oracle.p0uu(po, po, 0.99)
+    assert nv[0] == 3
+    D, diff, cnt = oracle.dmatrix(st, np.ones_like(po), np.nan)
+    assert (cnt == 0).all() and np.isnan(D).all()
+    assert (oracle.p0uu(po, po, np.nan)[2] == 0).all()
 
 
 def test_analyze_matches_numpy(oracle):
