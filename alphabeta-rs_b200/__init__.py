@@ -31,7 +31,7 @@ DBL_EPSILON = 2.220446049250313e-16
 SHRINK_ON_FAILED_CONTRACTION = 1
 NO_EARLY_EXIT_ON_STALL = 2
 
-TERM_SD, TERM_MAX_ITERS, TERM_STALLED, FIT_NAN = 1, 2, 3, -1
+TERM_SD, TERM_MAX_ITERS, TERM_STALLED, TERM_TARGET_COST, FIT_NAN = 1, 2, 3, 4, -1
 ERR_ARG, ERR_CUDA, ERR_TIME, ERR_NAN, ERR_TOO_LARGE, ERR_STATE = -1, -2, -3, -4, -5, -6
 
 

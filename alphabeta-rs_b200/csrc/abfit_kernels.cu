@@ -651,6 +651,9 @@ int launch_fit_boot(cudaStream_t st, const DevicePools &P, const WorkItem *items
                     int *err_flag, const BigScratch &big)
 {
     if (n_items <= 0) return 0;
+    if (getenv("ABFIT_DEV_VERBOSE"))
+        fprintf(stderr, "[abfit] k_fit_boot<BIG=%d>: %d blocks x 1 warp, %zu B smem/block\n", big.lm ? 1 : 0, n_items,
+                smem_bytes);
     if (big.lm) {
         if (int rc = prep_kernel(k_fit_boot<true>, smem_bytes)) return rc;
         k_fit_boot<true><<<n_items, 32, smem_bytes, st>>>(P, items, n_boot, best, pred, resid, resample_idx, vary,
@@ -674,6 +677,9 @@ int launch_fit_boot_gather(cudaStream_t st, const DevicePools &P, const WorkItem
 {
     if (n_items <= 0) return 0;
     if (int rc = prep_kernel(k_fit_boot_gather, smem_bytes)) return rc;
+    if (getenv("ABFIT_DEV_VERBOSE"))
+        fprintf(stderr, "[abfit] k_fit_boot_gather: %d blocks x 1 warp, %zu B smem/block%s\n", n_items, smem_bytes,
+                x_scratch ? " (vertices in global scratch)" : "");
     k_fit_boot_gather<<<n_items, 32, smem_bytes, st>>>(P, items, n_boot, best, pred, resid, resample_idx, vary,
                                                        static_cast<uint2 *>(idx_scratch), (long long)scratch_stride, nm,
                                                        rows_out, fits_out, evals_per_prob, err_flag, x_scratch);

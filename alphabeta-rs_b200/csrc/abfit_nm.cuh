@@ -277,6 +277,11 @@ __device__ __forceinline__ bool nm_advance(LaneNM &L, const LaneSimplex &S, cons
         } else if (L.iters >= P.max_iters) {
             L.status = ABFIT_TERM_MAX_ITERS;
             finish = true;
+        } else if (c[0] < -1.7976931348623157e308) {
+            // Executor: best_cost <= target_cost (-inf).  The sorted best equals the Executor's best_cost here: a
+            // -inf cost always replaces best_cost, and a NaN at position 0 is never the Executor's best.
+            L.status = ABFIT_TERM_TARGET_COST;
+            finish = true;
         } else {
             reflect_point(S, L.ord, L.xt);
             L.phase = PH_REFLECT;

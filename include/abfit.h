@@ -53,7 +53,12 @@ enum {
     ABFIT_TERM_STALLED = 3,   /* failed inside contraction left the simplex unchanged: every further
                                  iteration is identical, so the fit returns what the reference returns
                                  after max_iters; iters is reported as max_iters */
-    ABFIT_FIT_NAN = -1        /* best cost is NaN: the reference panics on best_param.unwrap() */
+    ABFIT_TERM_TARGET_COST = 4, /* best cost is -inf (argmin Executor: best_cost <= target_cost = -inf); tested
+                                   after the sd and max_iters tests, so those win when they fire too */
+    ABFIT_FIT_NAN = -1        /* best cost is NaN: the reference panics on best_param.unwrap().  This happens
+                                 exactly when vertex 0 of the start simplex costs NaN (a NaN never moves in the
+                                 stable sort, so it stays the best vertex); theta then holds that vertex, cost is
+                                 NaN and lse its penalty-free cost */
 };
 
 /* flags for fit/boot calls */

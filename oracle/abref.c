@@ -325,7 +325,10 @@ int abref_nelder_mead(const abref_problem *pb, const double simplex[20], int max
             status = ABREF_TERM_MAX_ITERS;
             break;
         }
-        if (best_cost <= -INFINITY) break;
+        if (best_cost <= -INFINITY) {
+            status = ABREF_TERM_TARGET_COST;
+            break;
+        }
 
         /* next_iter */
         double x0[4], xr[4];
@@ -387,6 +390,12 @@ int abref_nelder_mead(const abref_problem *pb, const double simplex[20], int max
         }
     }
 #undef UPDATE_BEST
+    if (!have_best) {
+        /* best_param stays None and the reference panics.  v[0] is the start's vertex 0 (its NaN cost never moves
+         * in the stable sort): report it with its NaN cost, as the library's records do (include/abfit.h) */
+        memcpy(best, v[0].x, sizeof best);
+        best_cost = v[0].c;
+    }
     memcpy(out->theta, best, sizeof best);
     out->cost = best_cost;
     out->iters = iters;
@@ -562,11 +571,11 @@ int abref_ab_neutral(const abref_problem *pb, int n_starts, const double *simpli
         }
     }
     for (int i = 0; i < n_starts; ++i) {
+        fits[i].lse = abref_lse(pb, fits[i].theta, flags);
         if (fits[i].status < 0) {
             rc = ABREF_ERR_NAN; /* :64,66 expect()/unwrap() panic */
             continue;
         }
-        fits[i].lse = abref_lse(pb, fits[i].theta, flags);
         if (fits[i].lse != fits[i].lse) rc = ABREF_ERR_NAN; /* :100 unwrap panic */
         if (arg < 0 || fits[i].lse < fits[arg].lse) arg = i;
     }

@@ -56,6 +56,7 @@ enum {
     ABREF_TERM_SD = 1,        /* sd of simplex costs < sd_tolerance */
     ABREF_TERM_MAX_ITERS = 2, /* iter >= max_iters */
     ABREF_TERM_STALLED = 3,   /* ABREF_NM_EARLY_EXIT_ON_STALL fired; iters reported = max_iters */
+    ABREF_TERM_TARGET_COST = 4, /* best_cost <= target_cost (-inf) */
     ABREF_ERR_NAN = -1,       /* reference would panic (NaN cost / best_param None) */
     ABREF_ERR_TIME = -2       /* t0>t1 or t0>t2 or outside i8: reference takes the matrix-inverse path */
 };

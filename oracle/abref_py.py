@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libabref.so")
 
 SHRINK_ON_FAILED_CONTRACTION, EARLY_EXIT_ON_STALL, FAST_DIVERGENCE, LITERAL_SORT = 1, 2, 4, 8
-TERM_SD, TERM_MAX_ITERS, TERM_STALLED, ERR_NAN, ERR_TIME = 1, 2, 3, -1, -2
+TERM_SD, TERM_MAX_ITERS, TERM_STALLED, TERM_TARGET_COST, ERR_NAN, ERR_TIME = 1, 2, 3, 4, -1, -2
 DBL_EPSILON = 2.220446049250313e-16
 
 

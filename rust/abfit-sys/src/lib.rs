@@ -34,6 +34,7 @@ pub const ABFIT_ERR_STATE: c_int = -6;
 pub const ABFIT_TERM_SD: i32 = 1;
 pub const ABFIT_TERM_MAX_ITERS: i32 = 2;
 pub const ABFIT_TERM_STALLED: i32 = 3;
+pub const ABFIT_TERM_TARGET_COST: i32 = 4;
 pub const ABFIT_FIT_NAN: i32 = -1;
 
 /// flags of the fit / bootstrap calls
