@@ -88,6 +88,11 @@ def _load() -> C.CDLL:
         "abfit_gen_start_simplices": (None, [u64, u64, i32, dbl, vp]),
         "abfit_gen_vary_vertices": (None, [u64, u64, i32, vp, vp]),
         "abfit_gen_resample_idx": (None, [u64, u64, i32, i32, vp]),
+        "abfit_gen_site_boot_counts": (None, [u64, u64, i32, i32, vp]),
+        "abfit_site_boot_batch": (C.c_int, [vp, PP, i32, vp, vp, vp, vp, i32, i64, vp, dbl, i64, vp, i32, u64, u64, vp, i32,
+                                            dbl, u32, vp, vp, vp, vp, vp]),
+        "abfit_site_boot_batch_device": (C.c_int, [vp, PP, i32, vp, vp, vp, vp, i32, i64, vp, dbl, i64, vp, i32, u64, u64, vp,
+                                                   i32, dbl, u32, vp, vp, vp, vp, vp]),
         "abfit_gen_vary_vertices_batch": (None, [u64, u64, i32, i32, vp, vp]),
         "abfit_device_count": (C.c_int, []),
         "abfit_alphabeta_batch_multi": (C.c_int, [vp, i32, vp, i32, i32, vp, i32, vp, u64, u64, vp, i32, i32, dbl, u32, vp, vp, vp, vp, vp, vp]),
@@ -168,7 +173,8 @@ EXPORTED_SYMBOLS = (
     "abfit_pedigree_free abfit_format_f64 abfit_steady_state abfit_write_pedigree abfit_write_analysis abfit_format_analysis "
     "abfit_write_npy_f64 abfit_write_metaprofile_results abfit_plot_metaplot abfit_plot_bootstrap "
     "abfit_sim_tree_build abfit_sim_tree_from_arrays abfit_sim_tree_info abfit_sim_tree_pairs abfit_sim_tree_thresholds "
-    "abfit_sim_tree_free abfit_sim_equilibrium abfit_simulate abfit_simulate_device"
+    "abfit_sim_tree_free abfit_sim_equilibrium abfit_simulate abfit_simulate_device "
+    "abfit_gen_site_boot_counts abfit_site_boot_batch abfit_site_boot_batch_device"
 ).split()
 
 
@@ -214,6 +220,13 @@ def gen_resample_idx(seed: int, problem_id: int, n_boot: int, n_pairs: int) -> n
     """residual resampling with replacement (src/boot_model.rs:43-48) -> int32 [n_boot,n_pairs]."""
     out = np.empty((n_boot, n_pairs), dtype=np.int32)
     _lib.abfit_gen_resample_idx(seed, problem_id, n_boot, n_pairs, _ptr(out))
+    return out
+
+
+def gen_site_boot_counts(seed: int, problem_key: int, n_boot: int, n_blocks: int) -> np.ndarray:
+    """multiplicity of every block of a window in every replicate of the site-block bootstrap, [n_boot, n_blocks] u32"""
+    out = np.zeros((n_boot, n_blocks), dtype=np.uint32)
+    _lib.abfit_gen_site_boot_counts(seed, problem_key, n_boot, n_blocks, _ptr(out))
     return out
 
 
@@ -531,6 +544,54 @@ class Context:
         )
         return {"D": D, "diff": diff, "cnt": cnt, "p0uu": p0uu, "methsum": methsum, "nvalid": nvalid,
                 "kernel_ms": (ms[0], ms[1]), "launches": launches.value}
+
+    # -- site-block bootstrap (include/abfit.h, abfit_site_boot_batch) ----------------------------
+    def _site_boot(self, fn, probs, pairs, inputs, S, L, seg_offsets, best, n_boot, seed, block_sites, thr,
+                   first_problem_id, problem_ids, max_iters, sd_tol, flags):
+        n_probs = len(probs)
+        pairs = np.ascontiguousarray(np.asarray(pairs)[:, :2], dtype=np.int32)
+        seg = np.ascontiguousarray(seg_offsets, dtype=np.int64)
+        best = np.ascontiguousarray(best, dtype=FIT_DTYPE).reshape(n_probs)
+        ids = None if problem_ids is None else np.ascontiguousarray(problem_ids, dtype=np.uint64)
+        total = sum(p.n_pairs for p in probs)
+        if pairs.shape[0] != total:
+            raise ValueError(f"pairs has {pairs.shape[0]} rows, the problems {total} pedigree rows")
+        if seg.shape != (n_probs + 1,):
+            raise ValueError(f"seg_offsets needs {n_probs + 1} entries, got {seg.size}")
+        if ids is not None and ids.shape != (n_probs,):
+            raise ValueError(f"problem_ids needs {n_probs} entries, got {ids.size}")
+        rows = np.empty((n_probs, n_boot, 7))
+        fits = np.zeros((n_probs, n_boot), dtype=FIT_DTYPE)
+        analysis = np.empty((n_probs, 32))
+        dstar = np.empty(total * n_boot)
+        nan_reps = np.zeros(n_probs, dtype=np.int32)
+        _check(fn(self._h, _pack_problems(probs), n_probs, _ptr(pairs), *inputs, S, L, _ptr(seg), thr, block_sites,
+                  _ptr(best), n_boot, seed, first_problem_id, _ptr(ids), max_iters, sd_tol, flags, _ptr(rows), _ptr(fits),
+                  _ptr(analysis), _ptr(dstar), _ptr(nan_reps)))
+        return {"rows": rows, "fits": fits, "analysis": analysis, "dstar": dstar, "nan_reps": nan_reps}
+
+    def site_bootstrap(self, probs: Sequence[Problem], pairs, status, posterior_max, meth_lvl, seg_offsets, best, n_boot,
+                       seed, block_sites, thr=0.99, first_problem_id=0, problem_ids=None, max_iters=1000,
+                       sd_tol=DBL_EPSILON, flags=0):
+        """Site-block bootstrap of fitted windows (abfit_site_boot_batch): window p = sites [seg_offsets[p],
+        seg_offsets[p+1]) of the [S, L] site arrays = problem p; pairs: the (i, j) sample columns of every pedigree row,
+        problems concatenated.  -> dict(rows [n_probs, n_boot, 7], fits, analysis [n_probs, 32], dstar (concatenated
+        [n_boot, n_pairs] blocks per problem), nan_reps [n_probs])"""
+        status = np.ascontiguousarray(status, dtype=np.uint8)
+        S, L = status.shape
+        post, meth = _f64(posterior_max, (S, L)), _f64(meth_lvl, (S, L))
+        return self._site_boot(_lib.abfit_site_boot_batch, probs, pairs, (_ptr(status), _ptr(post), _ptr(meth)), S, L,
+                               seg_offsets, best, n_boot, seed, block_sites, thr, first_problem_id, problem_ids, max_iters,
+                               sd_tol, flags)
+
+    def site_bootstrap_device(self, probs: Sequence[Problem], pairs, d_status: int, d_post: int, d_meth: int, S: int, L: int,
+                              seg_offsets, best, n_boot, seed, block_sites, thr=0.99, first_problem_id=0, problem_ids=None,
+                              max_iters=1000, sd_tol=DBL_EPSILON, flags=0):
+        """site_bootstrap() with the three [S, L] site arrays in device memory (ints: device pointers; the stream that
+        wrote them must be synchronised)"""
+        return self._site_boot(_lib.abfit_site_boot_batch_device, probs, pairs,
+                               (C.c_void_p(d_status), C.c_void_p(d_post), C.c_void_p(d_meth)), S, L, seg_offsets, best,
+                               n_boot, seed, block_sites, thr, first_problem_id, problem_ids, max_iters, sd_tol, flags)
 
     def batch(self, probs: Sequence[Problem]) -> "Batch":
         return Batch(self, probs)
@@ -997,7 +1058,7 @@ class SimTree:
 
 def design_study(ctxs, tree: SimTree, alpha, beta, weight=None, p0uu=None, *, L: int, n_replicates: int, n_starts=64,
                  n_boot=100, seed=0, missing_rate=0.0, thr=0.99, use_true_p0uu=True, max_iters_fit=10000,
-                 max_iters_boot=1000):
+                 max_iters_boot=1000, bootstrap="residual", block_sites=None):
     """How tightly does a design determine alpha and beta?  Simulates n_replicates independent data sets of L sites on
     `tree` and fits every one with alphabeta::run (multi-start fit + bootstrap):
       1. one simulation of n_replicates * L sites into device memory of ctxs[0] (replicate r = sites [r L, (r+1) L));
@@ -1008,6 +1069,9 @@ def design_study(ctxs, tree: SimTree, alpha, beta, weight=None, p0uu=None, *, L:
     use_true_p0uu: the problems' p0uu (and penalty target) is the simulated founder Pr(UU); otherwise the one the
     pipeline estimates from meth_lvl, mean over samples of 1 - mean(meth_lvl) = P(UU) + P(UM) / 2 (the reference's
     estimator, src/pedigree.rs:159-183), which is not P(UU).
+    bootstrap: "residual" (boot_model::run's resampling of pair residuals) or "sites": the site-block bootstrap
+    (Context.site_bootstrap_device, block_sites sites per block) of every replicate's simulated sites, behind a
+    fit_batch of the same starts; it runs on ctxs[0].
     Device memory: 17 bytes per sample-site of n_samples x n_replicates x L.
     -> dict(theta [R,4] best alpha, beta, weight, intercept; status [R] fit status (0 = ok); analysis [R,32]
     (abfit_analyze of the bootstrap); D [R,n_pairs]; p0uu [R] used; truth dict)"""
@@ -1018,6 +1082,10 @@ def design_study(ctxs, tree: SimTree, alpha, beta, weight=None, p0uu=None, *, L:
     R, S = int(n_replicates), tree.n_samples
     if R <= 0 or L <= 0 or S < 2 or tree.n_pairs == 0:
         raise ValueError("design_study needs n_replicates > 0, L > 0 and a tree with sampled pairs")
+    if bootstrap not in ("residual", "sites"):
+        raise ValueError("bootstrap must be 'residual' or 'sites'")
+    if bootstrap == "sites" and (block_sites is None or int(block_sites) < 1):
+        raise ValueError("bootstrap='sites' needs block_sites >= 1")
     dev = torch.device("cuda", ctxs[0].device)
     status = torch.empty((S, R * L), dtype=torch.uint8, device=dev)
     post = torch.empty((S, R * L), dtype=torch.float64, device=dev)
@@ -1027,11 +1095,19 @@ def design_study(ctxs, tree: SimTree, alpha, beta, weight=None, p0uu=None, *, L:
                             prm.p0uu, L=R * L, seed=seed, missing_rate=missing_rate)
     seg = np.arange(R + 1, dtype=np.int64) * L
     dm = ctxs[0].dmatrix_device(status.data_ptr(), post.data_ptr(), meth.data_ptr(), S, R * L, thr=thr, seg_offsets=seg)
-    del status, post, meth
+    if bootstrap == "residual":
+        del status, post, meth
     p0 = np.full(R, prm.p0uu) if use_true_p0uu else dm["p0uu"]
     probs = [Problem(tree.pedigree(dm["D"][r]), float(p0[r]), float(p0[r]), 1.0) for r in range(R)]
     sx = np.stack([gen_start_simplices(seed, r, n_starts, float(pb.pedigree[:, 3].max())) for r, pb in enumerate(probs)])
-    if len(ctxs) > 1:
+    if bootstrap == "sites":
+        fit = ctxs[0].fit_batch(probs, sx, max_iters=max_iters_fit, want_all=False)
+        pairs = np.tile(tree.pairs()[:, :2], (R, 1))
+        sb = ctxs[0].site_bootstrap_device(probs, pairs, status.data_ptr(), post.data_ptr(), meth.data_ptr(), S, R * L, seg,
+                                           fit.best, n_boot, seed, int(block_sites), thr=thr, max_iters=max_iters_boot)
+        del status, post, meth
+        res = {"best": fit.best, "status": fit.status, "analysis": sb["analysis"]}
+    elif len(ctxs) > 1:
         res = alphabeta_batch_multi(ctxs, probs, sx, n_boot, seed, max_iters_fit=max_iters_fit, max_iters_boot=max_iters_boot)
     else:
         res = ctxs[0].alphabeta_batch(probs, sx, n_boot, seed, max_iters_fit=max_iters_fit, max_iters_boot=max_iters_boot)

@@ -2,6 +2,11 @@
 // `alphabeta` binary (src/cli/alphabeta.rs:8-38, src/arguments.rs:96-114, src/alphabeta.rs:23-59), on top of libabfit.
 //
 //   alphabeta -n nodelist.txt -e edgelist.txt [-i 1000] [-p 0.99] [-o .] [--seed N] [--device 0 | --devices 0-7]
+//             [--site-bootstrap BLOCK_SITES]
+//
+// --site-bootstrap replaces the reference's residual bootstrap with the site-block bootstrap (abfit_site_boot_batch): the
+// replicates resample blocks of BLOCK_SITES consecutive sites of the methylome files, and the output files are written
+// from those rows.
 //
 // Differences that are deliberate: the random starts / resamples come from a seed (default 0xAB0B200,
 // `--seed` is an extra flag; the reference uses an unseeded thread_rng), the two progress bars advance per stage
@@ -12,6 +17,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <fstream>
+#include <sstream>
 #include <string>
 #include <sys/stat.h>
 #include <vector>
@@ -32,6 +39,68 @@ static std::string f64s(double v)
     return buf;
 }
 
+// The site arrays of the measured samples, read as abfit_pedigree_build reads them (node files relative to the CWD), and
+// the (i, j) samples of every pedigree row.  The site-block bootstrap needs every sample to list the same sites.
+static bool read_sites(const std::string &nodes, const std::string &edges, int32_t n_pairs, int32_t &S, int64_t &L,
+                       std::vector<uint8_t> &st, std::vector<double> &po, std::vector<double> &me, std::vector<int32_t> &pairs)
+{
+    std::vector<char> files(1 << 20);
+    std::vector<double> pr((size_t)n_pairs * 5);
+    int32_t np = 0;
+    if (abfit_pedigree_graph(nodes.c_str(), edges.c_str(), &S, files.data(), (int32_t)files.size(), &np, pr.data(), n_pairs) ||
+        np != n_pairs) {
+        std::printf("Error: %s\n", abfit_last_error());
+        return false;
+    }
+    pairs.resize((size_t)n_pairs * 2);
+    for (int32_t r = 0; r < n_pairs; ++r) {
+        pairs[2 * r] = (int32_t)pr[5 * r];
+        pairs[2 * r + 1] = (int32_t)pr[5 * r + 1];
+    }
+    std::istringstream names(std::string(files.data()));
+    std::string fn;
+    std::vector<std::vector<uint8_t>> s_st;
+    std::vector<std::vector<double>> s_po, s_me;
+    while (std::getline(names, fn)) {
+        std::ifstream f(fn, std::ios::binary);
+        if (!f) {
+            std::printf("Error: Could not open node file: %s\n", fn.c_str());
+            return false;
+        }
+        const std::string image((std::istreambuf_iterator<char>(f)), std::istreambuf_iterator<char>());
+        int64_t cap = 1, n = 0;
+        for (char ch : image) cap += ch == '\n';
+        s_st.emplace_back((size_t)cap);
+        s_po.emplace_back((size_t)cap);
+        s_me.emplace_back((size_t)cap);
+        if (abfit_parse_methylome_buffer(image.data(), (int64_t)image.size(), 0, 0, cap, nullptr, s_po.back().data(), s_st.back().data(),
+                                         s_me.back().data(), nullptr, nullptr, &n)) {
+            std::printf("Error: %s\n", abfit_last_error());
+            return false;
+        }
+        s_st.back().resize((size_t)n);
+        if (s_st.size() > 1 && s_st.back().size() != s_st[0].size()) {
+            std::printf("Error: --site-bootstrap: %s lists %lld sites, the first sample %lld; the site-block bootstrap needs "
+                        "every sample to list the same sites\n", fn.c_str(), (long long)n, (long long)s_st[0].size());
+            return false;
+        }
+    }
+    if ((int32_t)s_st.size() != S) {
+        std::printf("Error: --site-bootstrap: expected %d methylome files\n", S);
+        return false;
+    }
+    L = (int64_t)s_st[0].size();
+    st.resize((size_t)S * L);
+    po.resize((size_t)S * L);
+    me.resize((size_t)S * L);
+    for (int32_t s = 0; s < S; ++s) {
+        std::copy(s_st[s].begin(), s_st[s].begin() + L, st.begin() + (size_t)s * L);
+        std::copy(s_po[s].begin(), s_po[s].begin() + L, po.begin() + (size_t)s * L);
+        std::copy(s_me[s].begin(), s_me[s].begin() + L, me.begin() + (size_t)s * L);
+    }
+    return true;
+}
+
 int main(int argc, char **argv)
 {
     long iterations = 1000;
@@ -39,6 +108,7 @@ int main(int argc, char **argv)
     double filter = 0.99;
     unsigned long long seed = 0xAB0B200ull;
     int device = 0;
+    long long site_boot = 0;  // 0: the residual bootstrap of the reference
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto val = [&](const char *name) -> const char * {
@@ -55,6 +125,13 @@ int main(int argc, char **argv)
         else if (a == "-o" || a == "--output") output = val("--output");
         else if (a == "--seed") seed = std::strtoull(val("--seed"), nullptr, 0);
         else if (a == "--device") device = std::atoi(val("--device"));
+        else if (a == "--site-bootstrap") {
+            site_boot = std::atoll(val("--site-bootstrap"));
+            if (site_boot < 1) {
+                std::fprintf(stderr, "error: --site-bootstrap needs a block size of at least one site\n");
+                return 2;
+            }
+        }
         else if (a == "--devices") device = std::atoi(val("--devices"));  // one pedigree = one window: its starts and replicates stay on the first listed GPU
         else if (a == "-h" || a == "--help") {
             std::printf("Usage: alphabeta [OPTIONS]\n\nOptions:\n"
@@ -64,7 +141,8 @@ int main(int argc, char **argv)
                         "  -p, --posterior-max-filter <P> Minimum posterior probability for a basepair read [default: 0.99]\n"
                         "  -o, --output <OUTPUT>          Output directory, must exist [default: .]\n"
                         "      --seed <SEED>              Seed of the random starts and resamples [default: 0xAB0B200]\n"
-                        "      --device <N>               CUDA device [default: 0]\n");
+                        "      --device <N>               CUDA device [default: 0]\n"
+                        "      --site-bootstrap <SITES>   Bootstrap by resampling blocks of SITES consecutive sites instead of pair residuals\n");
             return 0;
         } else {
             std::fprintf(stderr, "error: unexpected argument '%s' found\n", a.c_str());
@@ -119,8 +197,28 @@ int main(int argc, char **argv)
     int32_t status = 0;
     progress::Bar pb_neutral("ABNeutral", (unsigned long long)n, false), pb_boot("BootModel", (unsigned long long)n, false);  // src/progress.rs:5-23
     pb_neutral.tick();
-    const int rc = abfit_alphabeta_batch(ctx, &prob, 1, n, simplices.data(), n, idx.data(), seed, 0, 10000, 1000, DBL_EPSILON, 0,
-                                         &best, pred.data(), resid.data(), &status, rows_out.data(), analysis.data());
+    int rc = 0;
+    if (site_boot > 0) {
+        // fit as abfit_alphabeta_batch does, then the site-block bootstrap on the methylomes' own sites
+        int32_t S = 0;
+        int64_t L = 0;
+        std::vector<uint8_t> st;
+        std::vector<double> po, me;
+        std::vector<int32_t> pairs;
+        if (!read_sites(nodes, edges, n_pairs, S, L, st, po, me, pairs)) return 1;
+        rc = abfit_fit_batch(ctx, &prob, 1, n, simplices.data(), 10000, DBL_EPSILON, 0, &best, nullptr, nullptr, nullptr, &status);
+        const int64_t seg[2] = {0, L};
+        int32_t nan_reps = 0;
+        if (!rc && !status)
+            rc = abfit_site_boot_batch(ctx, &prob, 1, pairs.data(), st.data(), po.data(), me.data(), S, L, seg, filter, site_boot,
+                                       &best, n, seed, 0, nullptr, 1000, DBL_EPSILON, 0, rows_out.data(), nullptr, analysis.data(),
+                                       nullptr, &nan_reps);
+        if (!rc && nan_reps)
+            std::printf("Site bootstrap: %d of %d replicates left a pair without valid sites (NaN rows)\n", nan_reps, n);
+    } else {
+        rc = abfit_alphabeta_batch(ctx, &prob, 1, n, simplices.data(), n, idx.data(), seed, 0, 10000, 1000, DBL_EPSILON, 0, &best,
+                                   pred.data(), resid.data(), &status, rows_out.data(), analysis.data());
+    }
     if (rc || status) {
         std::printf("Error: Model failed: %s\n", rc ? abfit_last_error() : "NaN in the pedigree or in every fit (the reference panics here)");
         return 1;

@@ -6,6 +6,7 @@
 //
 //   metaprofile -m <methylome dir> -g <annotation> [-w 5] [-s 0] [-o .] [-a] [-c 2048] [-i] [--name N]
 //               [--cutoff-gene-length] [--iterations 100] [--seed N] [--device 0 | --devices 0-7] [--write-windows]
+//               [--site-bootstrap BLOCK_SITES]
 //               [alphabeta --nodes <nodelist> --edges <edgelist>]
 //
 // Files written (formats of the reference): distribution_<file>, distributions.txt, steady_state_methylation.txt,
@@ -130,6 +131,7 @@ int main(int argc, char **argv)
     unsigned long long seed = 0xAB0B200ull;
     int device = 0;
     std::vector<int> devices;  // --devices 0-7 / 0,2,5: windows sharded over several GPUs (abfit_alphabeta_batch_multi)
+    long long site_boot = 0;   // --site-bootstrap N: site-block bootstrap of N-site blocks (0: the residual bootstrap)
     for (int i = 1; i < argc; ++i) {
         const std::string a = argv[i];
         auto val = [&]() -> const char * {
@@ -158,6 +160,13 @@ int main(int argc, char **argv)
         else if (a == "--seed") seed = std::strtoull(val(), nullptr, 0);
         else if (a == "--device") device = std::atoi(val());
         else if (a == "--write-windows") write_windows = true;
+        else if (a == "--site-bootstrap") {
+            site_boot = std::atoll(val());
+            if (site_boot < 1) {
+                std::fprintf(stderr, "error: --site-bootstrap needs a block size of at least one site\n");
+                return 2;
+            }
+        }
         else if (a == "--devices") {
             const std::string v = val();
             size_t pos = 0;
@@ -178,6 +187,10 @@ int main(int argc, char **argv)
     }
     if (methylome.empty() || genome.empty()) {
         std::fprintf(stderr, "error: the following required arguments were not provided:\n  --methylome <METHYLOME>\n  --genome <GENOME>\n");
+        return 2;
+    }
+    if (site_boot > 0 && devices.size() > 1) {
+        std::fprintf(stderr, "error: --site-bootstrap runs on one device; --devices names %zu\n", devices.size());
         return 2;
     }
     std::printf("Starting run %s\n", name.c_str());
@@ -483,13 +496,6 @@ int main(int argc, char **argv)
         std::printf("Error: Error while building pedigree: the nodelist has fewer than two measured samples\n");
         return 1;
     }
-    if (devices.empty()) devices.push_back(device);
-    std::vector<abfit_ctx *> ctxs(devices.size(), nullptr);
-    for (size_t d = 0; d < devices.size(); ++d)
-        if (abfit_ctx_create(devices[d], &ctxs[d])) {
-            std::printf("Error: %s\n", abfit_last_error());
-            return 1;
-        }
     // Windows whose samples all list the same number of sites ("regular") go into ONE divergence call.  A window whose
     // samples list different numbers of sites is kept, as in the reference: DMatrix::from prints "Lengths do not match, all
     // bets are off" and leaves D = 0 for every pair of unequal length (src/pedigree.rs:222-230); pairs of equal length are
@@ -520,13 +526,26 @@ int main(int argc, char **argv)
             reg_of.push_back(-1);
         }
     }
+    if (site_boot > 0)  // DMatrix::from sets D = 0 for pairs of unequal length: a site bootstrap of such a window is undefined
+        for (size_t k = 0; k < usable.size(); ++k)
+            if (reg_of[k] < 0) {
+                std::printf("Error: --site-bootstrap: the samples of window %d list different numbers of sites\n", usable[k]);
+                return 1;
+            }
+    if (devices.empty()) devices.push_back(device);
+    std::vector<abfit_ctx *> ctxs(devices.size(), nullptr);
+    for (size_t d = 0; d < devices.size(); ++d)
+        if (abfit_ctx_create(devices[d], &ctxs[d])) {
+            std::printf("Error: %s\n", abfit_last_error());
+            return 1;
+        }
     const int64_t L = seg.back();
     const int W = (int)usable.size(), WR = (int)reg_windows.size();
     const size_t P = (size_t)S * (S - 1) / 2;
     std::vector<double> D((size_t)std::max(W, 1) * std::max<size_t>(P, 1), 0.0), p0uu(std::max(W, 1));
+    std::vector<uint8_t> st((size_t)S * L);  // the regular windows' sites (kept for --site-bootstrap)
+    std::vector<double> po((size_t)S * L), me((size_t)S * L);
     {
-        std::vector<uint8_t> st((size_t)S * L);
-        std::vector<double> po((size_t)S * L), me((size_t)S * L);
         parallel_for((size_t)S * 8, [&](size_t job) {  // eight slices of the window list per sample
             const size_t s = job / 8, part = job % 8;
             const Sample &A = samples[sample_of[s]];
@@ -653,9 +672,48 @@ int main(int argc, char **argv)
     // call, so the bar stands at the windows prepared so far while the GPUs work and jumps to the end afterwards
     progress::Bar pb("Progress ", (unsigned long long)n_total, true);
     pb.set((unsigned long long)(n_total - F));
-    if (F > 0 && abfit_alphabeta_batch_multi(ctxs.data(), (int32_t)ctxs.size(), probs.data(), F, n, simplices.get(), n, nullptr, seed,
-                                             0, ids.data(), 10000, 1000, DBL_EPSILON, 0, best.data(), nullptr, nullptr,
-                                             status.data(), rows.data(), analysis.data())) {
+    if (F > 0 && site_boot > 0) {
+        // the fit of abfit_alphabeta_batch, then the site-block bootstrap of every fitted window on its own sites (the
+        // fitted windows' sites copied next to each other: window f = problem f)
+        std::vector<int64_t> fseg(F + 1, 0);
+        for (int f = 0; f < F; ++f) {
+            const int r = reg_of[fitted[f]];
+            fseg[f + 1] = fseg[f] + seg[r + 1] - seg[r];
+        }
+        const int64_t LF = fseg[F];
+        std::vector<uint8_t> fst((size_t)S * LF);
+        std::vector<double> fpo((size_t)S * LF), fme((size_t)S * LF);
+        parallel_for((size_t)S, [&](size_t s) {
+            for (int f = 0; f < F; ++f) {
+                const int r = reg_of[fitted[f]];
+                const int64_t len = seg[r + 1] - seg[r];
+                std::copy_n(st.begin() + s * L + seg[r], len, fst.begin() + s * LF + fseg[f]);
+                std::copy_n(po.begin() + s * L + seg[r], len, fpo.begin() + s * LF + fseg[f]);
+                std::copy_n(me.begin() + s * L + seg[r], len, fme.begin() + s * LF + fseg[f]);
+            }
+        });
+        std::vector<int32_t> rp((size_t)F * n_pairs * 2);
+        for (int f = 0; f < F; ++f)
+            for (int q = 0; q < n_pairs; ++q) {
+                rp[((size_t)f * n_pairs + q) * 2] = (int32_t)pairs[5 * q];
+                rp[((size_t)f * n_pairs + q) * 2 + 1] = (int32_t)pairs[5 * q + 1];
+            }
+        std::vector<int32_t> nan_reps(F);
+        if (abfit_fit_batch(ctxs[0], probs.data(), F, n, simplices.get(), 10000, DBL_EPSILON, 0, best.data(), nullptr, nullptr,
+                            nullptr, status.data()) ||
+            abfit_site_boot_batch(ctxs[0], probs.data(), F, rp.data(), fst.data(), fpo.data(), fme.data(), S, LF, fseg.data(), 0.99,
+                                  site_boot, best.data(), n, seed, 0, ids.data(), 1000, DBL_EPSILON, 0, rows.data(), nullptr,
+                                  analysis.data(), nullptr, nan_reps.data())) {
+            std::printf("Error: %s\n", abfit_last_error());
+            return 1;
+        }
+        for (int f = 0; f < F; ++f)
+            if (nan_reps[f])
+                std::printf("Site bootstrap: window %d: %d of %d replicates left a pair without valid sites (NaN rows)\n",
+                            usable[fitted[f]], nan_reps[f], n);
+    } else if (F > 0 && abfit_alphabeta_batch_multi(ctxs.data(), (int32_t)ctxs.size(), probs.data(), F, n, simplices.get(), n, nullptr,
+                                                    seed, 0, ids.data(), 10000, 1000, DBL_EPSILON, 0, best.data(), nullptr, nullptr,
+                                                    status.data(), rows.data(), analysis.data())) {
         std::printf("Error: %s\n", abfit_last_error());
         return 1;
     }

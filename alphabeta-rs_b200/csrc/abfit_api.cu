@@ -1517,6 +1517,278 @@ int abfit_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const doubl
                            cnt_out, p0uu_out, methsum_out, nvalid_out, kernel_ms, launches_out);
 }
 
+// ---------------------------------------------------------------------------------------
+// site-block bootstrap: per-block partial sums (the observed-divergence path over a list of block windows) -> D* of
+// every replicate (k_siteboot_dstar) -> the bootstrap refit kernels on the given D* (DGIVEN instantiations)
+// ---------------------------------------------------------------------------------------
+void abfit_gen_site_boot_counts(uint64_t seed, uint64_t problem_key, int32_t n_boot, int32_t n_blocks, uint32_t *counts_out)
+{
+    if (!counts_out || n_boot <= 0 || n_blocks <= 0) return;
+    std::fill(counts_out, counts_out + (size_t)n_boot * n_blocks, 0u);
+    for (int32_t b = 0; b < n_boot; ++b)
+        for (int32_t d = 0; d < n_blocks; ++d)
+            ++counts_out[(size_t)b * n_blocks + site_boot_block(seed, problem_key, (uint64_t)b, (uint64_t)d, n_blocks)];
+}
+
+static int site_boot_impl(abfit_ctx *ctx, bool device_inputs, const abfit_problem *probs, int32_t n_probs,
+                          const int32_t *pairs, const uint8_t *status, const double *posterior_max, const double *meth_lvl,
+                          int32_t S, int64_t L, const int64_t *seg, double thr, int64_t block_sites, const abfit_fit *best,
+                          int32_t n_boot, uint64_t seed, uint64_t first_problem_id, const uint64_t *problem_ids,
+                          int32_t max_iters, double sd_tol, uint32_t flags, double *rows_out, abfit_fit *fits_out,
+                          double *analysis_out, double *dstar_out, int32_t *nan_reps_out)
+{
+    // every refusal that needs no device comes first
+    if (block_sites < 1 || block_sites >= ((int64_t)1 << 31)) {
+        set_error("site bootstrap: block_sites must lie in [1, 2^31)");
+        return ABFIT_ERR_ARG;
+    }
+    if (!probs || n_probs <= 0 || !pairs || !seg || !best || !rows_out || n_boot <= 0 || max_iters < 0 || !status ||
+        !posterior_max || !meth_lvl || S < 2 || S > 65535 || L < 0) {
+        set_error("site bootstrap: missing or out-of-range argument");
+        return ABFIT_ERR_ARG;
+    }
+    if (seg[0] < 0 || seg[n_probs] > L) {
+        set_error("site bootstrap: seg_offsets outside [0, L]");
+        return ABFIT_ERR_ARG;
+    }
+    std::vector<long long> blk_off((size_t)n_probs + 1, 0);
+    std::vector<int64_t> bseg;
+    for (int p = 0; p < n_probs; ++p) {
+        const int64_t len = seg[p + 1] - seg[p];
+        if (len <= 0) {
+            set_error("site bootstrap: window " + std::to_string(p) + " has no sites");
+            return ABFIT_ERR_ARG;
+        }
+        const int64_t nb = (len + block_sites - 1) / block_sites;
+        if (nb > INT32_MAX) {
+            set_error("site bootstrap: window " + std::to_string(p) + " has 2^31 blocks or more");
+            return ABFIT_ERR_ARG;
+        }
+        for (int64_t k = 0; k < nb; ++k) bseg.push_back(seg[p] + k * block_sites);
+        blk_off[p + 1] = blk_off[p] + nb;
+    }
+    bseg.push_back(seg[n_probs]);
+    const int64_t n_blk = blk_off[n_probs];
+    if (n_blk > INT32_MAX) {
+        set_error("site bootstrap: 2^31 blocks or more in one call");
+        return ABFIT_ERR_ARG;
+    }
+    const int64_t P = (int64_t)S * (S - 1) / 2;
+    int64_t total_pairs = 0;
+    int32_t max_rows = 0;
+    for (int p = 0; p < n_probs; ++p) {
+        if (probs[p].n_pairs <= 0) {
+            set_error("site bootstrap: problem " + std::to_string(p) + " has no pedigree rows");
+            return ABFIT_ERR_ARG;
+        }
+        total_pairs += probs[p].n_pairs;
+        max_rows = std::max(max_rows, probs[p].n_pairs);
+    }
+    std::vector<int32_t> row_pair((size_t)total_pairs);
+    for (int64_t r = 0; r < total_pairs; ++r) {
+        int64_t i = pairs[2 * r], j = pairs[2 * r + 1];
+        if (i < 0 || j < 0 || i >= S || j >= S || i == j) {
+            set_error("site bootstrap: pedigree row " + std::to_string(r) + " names no pair of the S samples");
+            return ABFIT_ERR_ARG;
+        }
+        if (i > j) std::swap(i, j);
+        row_pair[(size_t)r] = (int32_t)(i * S - i * (i + 1) / 2 + (j - i - 1));  // pair order (0,1),(0,2)...
+    }
+    if (!ctx) {
+        set_error("site bootstrap: no context");
+        return ABFIT_ERR_ARG;
+    }
+    ABFIT_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    // the pedigrees are compiled (and refused) before the partial sums are computed
+    abfit_batch *b = nullptr;
+    if (int rc = workspace(ctx, probs, n_probs, &b)) return rc;
+
+    // device memory: the partials stay resident; the divergence's u64 outputs are produced a chunk of blocks at a time
+    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(n_blk, ((int64_t)256 << 20) / (P * 24)));
+    const size_t n_in = device_inputs ? 0 : (size_t)S * (size_t)L * 17;
+    const size_t need = (size_t)n_blk * P * 8 + (size_t)chunk * (P * 24 + S * 16) + (size_t)n_blk * n_boot * 4 +
+                        (size_t)total_pairs * n_boot * 8 + n_in + (size_t)S * (size_t)L * 3 / 8 + ((size_t)64 << 20);
+    {
+        size_t fr = 0, tot = 0;
+        ABFIT_CUDA(cudaMemGetInfo(&fr, &tot));
+        if (need > fr) {
+            set_error("site bootstrap: " + std::to_string(n_blk) + " blocks x " + std::to_string(P) +
+                      " pairs need about " + std::to_string(need >> 20) + " MiB of device memory, " +
+                      std::to_string(fr >> 20) + " MiB are free");
+            return ABFIT_ERR_TOO_LARGE;
+        }
+    }
+    DevBuf<uint2> d_part;
+    if (int rc = d_part.ensure((size_t)n_blk * P)) return rc;
+    {
+        DevBuf<uint8_t> in_status;
+        DevBuf<double> in_post, in_meth;
+        if (!device_inputs && L > 0) {
+            const size_t n = (size_t)S * (size_t)L;
+            if (int rc = in_status.ensure(n)) return rc;
+            if (int rc = in_post.ensure(n)) return rc;
+            if (int rc = in_meth.ensure(n)) return rc;
+            ABFIT_CUDA(cudaMemcpyAsync(in_status.p, status, n, cudaMemcpyHostToDevice, st));
+            ABFIT_CUDA(cudaMemcpyAsync(in_post.p, posterior_max, n * 8, cudaMemcpyHostToDevice, st));
+            ABFIT_CUDA(cudaMemcpyAsync(in_meth.p, meth_lvl, n * 8, cudaMemcpyHostToDevice, st));
+            status = in_status.p;
+            posterior_max = in_post.p;
+            meth_lvl = in_meth.p;
+        }
+        DevBuf<double> t_D, t_ms;
+        DevBuf<unsigned long long> t_diff, t_cnt;
+        DevBuf<long long> t_nv;
+        if (int rc = t_D.ensure((size_t)chunk * P)) return rc;
+        if (int rc = t_diff.ensure((size_t)chunk * P)) return rc;
+        if (int rc = t_cnt.ensure((size_t)chunk * P)) return rc;
+        if (int rc = t_ms.ensure((size_t)chunk * S)) return rc;
+        if (int rc = t_nv.ensure((size_t)chunk * S)) return rc;
+        // the fused / two-pass choice is made once for the whole block list, as one abfit_divergence call would
+        const int long_windows = div_long_windows(bseg.data(), (int)n_blk) ? 1 : 0;
+        for (int64_t c0 = 0; c0 < n_blk; c0 += chunk) {
+            const int W = (int)std::min<int64_t>(chunk, n_blk - c0);
+            int launches = 0;
+            if (int rc = run_divergence(st, status, posterior_max, meth_lvl, S, L, bseg.data() + c0, W, thr, t_D.p, t_diff.p,
+                                        t_cnt.p, t_ms.p, t_nv.p, nullptr, &launches, nullptr, &ctx->div_arena, long_windows))
+                return rc;
+            if (int rc = launch_siteboot_pack(st, t_diff.p, t_cnt.p, (int64_t)W * P, d_part.p + (size_t)c0 * P)) return rc;
+        }
+        ABFIT_CUDA(cudaStreamSynchronize(st));  // the temporaries are freed at the end of this scope
+    }
+
+    // the mapping abfit_boot_batch's planner picks for these pedigrees: warp-per-fit, else the stored-D* tile
+    const int n_sm = ctx->prop.multiProcessorCount;
+    std::vector<WorkItem> items = b->shape.wide ? make_items_wide(b->hp, n_boot, n_sm, false)
+                                                : make_items(b->hp, n_boot, n_sm, 1, false);
+    std::vector<SiteBootItem> ditems;
+    {
+        int64_t off = 0;
+        for (int p = 0; p < n_probs; ++p) {
+            const int np = probs[p].n_pairs;
+            for (int r0 = 0; r0 < np; r0 += SB_THREADS) {
+                SiteBootItem it{};
+                it.prob = p;
+                it.r0 = r0;
+                it.n_rows = std::min(SB_THREADS, np - r0);
+                it.n_pairs = np;
+                it.pair_off = off;
+                it.blk0 = blk_off[p];
+                it.n_blk = (int32_t)(blk_off[p + 1] - blk_off[p]);
+                ditems.push_back(it);
+            }
+            off += np;
+        }
+    }
+    DevBuf<WorkItem> d_items;
+    DevBuf<SiteBootItem> d_ditems;
+    DevBuf<long long> d_blk_off;
+    DevBuf<int32_t> d_row_pair;
+    DevBuf<uint32_t> d_counts;
+    DevBuf<double> d_dstar, d_rows, d_tile, d_an, d_an_scratch;
+    DevBuf<uint8_t> d_nan;
+    DevBuf<abfit_fit> d_fits;
+    if (int rc = d_items.ensure(items.size())) return rc;
+    if (int rc = d_ditems.ensure(ditems.size())) return rc;
+    if (int rc = d_blk_off.ensure(blk_off.size())) return rc;
+    if (int rc = d_row_pair.ensure(row_pair.size())) return rc;
+    if (int rc = d_counts.ensure((size_t)n_blk * n_boot)) return rc;
+    if (int rc = d_dstar.ensure((size_t)total_pairs * n_boot)) return rc;
+    if (int rc = d_nan.ensure((size_t)n_probs * n_boot)) return rc;
+    if (int rc = d_rows.ensure((size_t)n_probs * n_boot * 7)) return rc;
+    if (int rc = d_fits.ensure((size_t)n_probs * n_boot)) return rc;
+    if (int rc = b->d_best.ensure(n_probs)) return rc;
+    if (int rc = b->d_vary.ensure((size_t)n_probs * n_boot * 16)) return rc;
+    if (!b->shape.wide)
+        if (int rc = d_tile.ensure((items.size() + 1) * (size_t)b->hp.max_pairs * 32)) return rc;
+    const bool dev_stats = analysis_out && n_boot >= 2;
+    if (dev_stats) {
+        if (int rc = d_an.ensure((size_t)n_probs * 32)) return rc;
+        if (int rc = d_an_scratch.ensure((size_t)n_probs * 8 * n_boot)) return rc;
+    }
+    BigScratch big;
+    if (!b->shape.wide)
+        if (int rc = big_scratch(b, std::max<size_t>(items.size(), 1), big)) return rc;
+    const unsigned long long *d_ids = nullptr;
+    if (problem_ids) {
+        if (int rc = b->d_ids.ensure(n_probs)) return rc;
+        ABFIT_CUDA(cudaMemcpyAsync(b->d_ids.p, problem_ids, (size_t)n_probs * 8, cudaMemcpyHostToDevice, st));
+        d_ids = b->d_ids.p;
+    }
+    if (!items.empty())
+        ABFIT_CUDA(cudaMemcpyAsync(d_items.p, items.data(), items.size() * sizeof(WorkItem), cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemcpyAsync(d_ditems.p, ditems.data(), ditems.size() * sizeof(SiteBootItem), cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemcpyAsync(d_blk_off.p, blk_off.data(), blk_off.size() * 8, cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemcpyAsync(d_row_pair.p, row_pair.data(), row_pair.size() * 4, cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemcpyAsync(b->d_best.p, best, (size_t)n_probs * sizeof(abfit_fit), cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_counts.p, 0, (size_t)n_blk * n_boot * 4, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_nan.p, 0, (size_t)n_probs * n_boot, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_rows.p, 0xFF, (size_t)n_probs * n_boot * 7 * 8, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_fits.p, 0xFF, (size_t)n_probs * n_boot * sizeof(abfit_fit), st));
+    ABFIT_CUDA(cudaMemsetAsync(b->d_evals_boot.p, 0, (size_t)n_probs * 8, st));
+    if (int rc = launch_gen_vary(st, seed, first_problem_id, d_ids, n_probs, n_boot, b->d_best.p, b->d_vary.p)) return rc;
+    if (int rc = launch_siteboot_counts(st, seed, first_problem_id, d_ids, d_blk_off.p, n_probs, n_boot, n_blk, d_counts.p)) return rc;
+    if (int rc = launch_siteboot_dstar(st, d_ditems.p, (int)ditems.size(), n_boot, d_part.p, P, d_counts.p, d_row_pair.p,
+                                       d_dstar.p, d_nan.p))
+        return rc;
+    const NMParams nm = nm_params(max_iters, sd_tol, flags);
+    if (b->shape.wide) {
+        if (int rc = launch_fit_boot_wide_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar.p,
+                                                b->d_vary.p, nm, d_rows.p, d_fits.p, b->d_evals_boot.p, b->shape.smem_wide))
+            return rc;
+    } else if (int rc = launch_fit_boot_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar.p,
+                                              b->d_vary.p, d_tile.p, (int64_t)b->hp.max_pairs * 32, nm, d_rows.p, d_fits.p,
+                                              b->d_evals_boot.p, b->shape.smem_boot, big)) {
+        return rc;
+    }
+    if (dev_stats) {
+        if (int rc = launch_analyze(st, d_rows.p, n_probs, n_boot, d_an.p, d_an_scratch.p)) return rc;
+        ABFIT_CUDA(cudaMemcpyAsync(analysis_out, d_an.p, (size_t)n_probs * 32 * 8, cudaMemcpyDeviceToHost, st));
+    }
+    std::vector<uint8_t> nan_rep((size_t)n_probs * n_boot);
+    ABFIT_CUDA(cudaMemcpyAsync(rows_out, d_rows.p, (size_t)n_probs * n_boot * 7 * 8, cudaMemcpyDeviceToHost, st));
+    if (fits_out)
+        ABFIT_CUDA(cudaMemcpyAsync(fits_out, d_fits.p, (size_t)n_probs * n_boot * sizeof(abfit_fit), cudaMemcpyDeviceToHost, st));
+    if (dstar_out)
+        ABFIT_CUDA(cudaMemcpyAsync(dstar_out, d_dstar.p, (size_t)total_pairs * n_boot * 8, cudaMemcpyDeviceToHost, st));
+    ABFIT_CUDA(cudaMemcpyAsync(nan_rep.data(), d_nan.p, nan_rep.size(), cudaMemcpyDeviceToHost, st));
+    ABFIT_CUDA(cudaStreamSynchronize(st));
+    if (nan_reps_out)
+        for (int p = 0; p < n_probs; ++p) {
+            int32_t n = 0;
+            for (int k = 0; k < n_boot; ++k) n += nan_rep[(size_t)p * n_boot + k];
+            nan_reps_out[p] = n;
+        }
+    if (analysis_out && !dev_stats)
+        for (int p = 0; p < n_probs; ++p) abfit_analyze(rows_out + (size_t)p * n_boot * 7, n_boot, analysis_out + (size_t)p * 32);
+    return 0;
+}
+
+int abfit_site_boot_batch(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_probs, const int32_t *pairs,
+                          const uint8_t *status, const double *posterior_max, const double *meth_lvl, int32_t S, int64_t L,
+                          const int64_t *seg_offsets, double thr, int64_t block_sites, const abfit_fit *best,
+                          int32_t n_boot, uint64_t seed, uint64_t first_problem_id, const uint64_t *problem_ids,
+                          int32_t max_iters, double sd_tol, uint32_t flags, double *rows_out, abfit_fit *fits_out,
+                          double *analysis_out, double *dstar_out, int32_t *nan_reps_out)
+{
+    return site_boot_impl(ctx, false, probs, n_probs, pairs, status, posterior_max, meth_lvl, S, L, seg_offsets, thr,
+                          block_sites, best, n_boot, seed, first_problem_id, problem_ids, max_iters, sd_tol, flags, rows_out,
+                          fits_out, analysis_out, dstar_out, nan_reps_out);
+}
+
+int abfit_site_boot_batch_device(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_probs, const int32_t *pairs,
+                                 const uint8_t *d_status, const double *d_posterior_max, const double *d_meth_lvl, int32_t S,
+                                 int64_t L, const int64_t *seg_offsets, double thr, int64_t block_sites,
+                                 const abfit_fit *best, int32_t n_boot, uint64_t seed, uint64_t first_problem_id,
+                                 const uint64_t *problem_ids, int32_t max_iters, double sd_tol, uint32_t flags,
+                                 double *rows_out, abfit_fit *fits_out, double *analysis_out, double *dstar_out,
+                                 int32_t *nan_reps_out)
+{
+    return site_boot_impl(ctx, true, probs, n_probs, pairs, d_status, d_posterior_max, d_meth_lvl, S, L, seg_offsets, thr,
+                          block_sites, best, n_boot, seed, first_problem_id, problem_ids, max_iters, sd_tol, flags, rows_out,
+                          fits_out, analysis_out, dstar_out, nan_reps_out);
+}
+
 int abfit_simulate(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site, int64_t L,
                    uint8_t *status, double *posterior_max, double *meth_lvl)
 {

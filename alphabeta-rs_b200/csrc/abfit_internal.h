@@ -62,6 +62,15 @@ int launch_fit_boot_wide(cudaStream_t st, const DevicePools &P, const WorkItem *
                          const double *vary, double *dstar_scratch, int64_t scratch_stride, NMParams nm,
                          double *rows_out, abfit_fit *fits_out, unsigned long long *evals_per_prob, size_t smem_bytes,
                          int *err_flag);
+// site-block bootstrap refits (abfit_site_boot_batch): the same kernels fitting a given D* matrix
+// dstar[pair_off * n_boot + b * n_pairs + i]; a replicate with a NaN D* is not fitted (NaN row, ABFIT_FIT_NAN)
+int launch_fit_boot_given(cudaStream_t st, const DevicePools &P, const WorkItem *items, int n_items, int n_boot,
+                          const abfit_fit *best, const double *dstar, const double *vary, double *tile_scratch,
+                          int64_t scratch_stride, NMParams nm, double *rows_out, abfit_fit *fits_out,
+                          unsigned long long *evals_per_prob, size_t smem_bytes, const BigScratch &big);
+int launch_fit_boot_wide_given(cudaStream_t st, const DevicePools &P, const WorkItem *items, int n_items, int n_boot,
+                               const abfit_fit *best, const double *dstar, const double *vary, NMParams nm,
+                               double *rows_out, abfit_fit *fits_out, unsigned long long *evals_per_prob, size_t smem_bytes);
 int launch_cost_batch(cudaStream_t st, const DevicePools &P, const WorkItem *items, int n_items,
                       const double *theta, double *cost_out, double *lse_out, size_t smem_bytes, bool d_in_shared,
                       const BigScratch &big);
@@ -106,6 +115,25 @@ int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_pos
 // two-pass path sum meth_lvl in different trees, so a call that is split over devices decides this once, for all of
 // its windows, and passes the answer to every shard: each window then gets the bits one device gives it.
 bool div_long_windows(const int64_t *h_seg, int W);
+
+// ---- site-block bootstrap (abfit_siteboot.cu) ---------------------------------------------
+constexpr int SB_THREADS = 128;  // pedigree rows per block of k_siteboot_dstar
+constexpr int SB_TB = 16;        // replicates per block (u64 accumulators per thread: 2 * SB_TB)
+constexpr int SB_KC = 256;       // blocks of counts staged in shared memory at a time
+struct SiteBootItem {
+    int32_t prob, r0, n_rows, n_pairs;  // pedigree rows [r0, r0 + n_rows) of window prob
+    int64_t pair_off;                   // first pedigree row of the window in the concatenated rows
+    int64_t blk0;                       // first block of the window in the block list
+    int32_t n_blk, pad;
+};
+// partials[k][P] = (diff, cnt) of block k from the u64 sums of run_divergence
+int launch_siteboot_pack(cudaStream_t st, const unsigned long long *diff, const unsigned long long *cnt, int64_t n, uint2 *out);
+// counts[blk_off[p] * n_boot + b * n_blk + k]: multiplicity of block k of window p in replicate b (counts zeroed first)
+int launch_siteboot_counts(cudaStream_t st, uint64_t seed, uint64_t first_problem_id, const unsigned long long *ids,
+                           const long long *blk_off, int n_probs, int n_boot, int64_t n_blk_total, uint32_t *counts);
+// dstar[pair_off * n_boot + b * n_pairs + r]; nan_rep[p * n_boot + b] = 1 when a pair of the replicate has no site
+int launch_siteboot_dstar(cudaStream_t st, const SiteBootItem *items, int n_items, int n_boot, const uint2 *partials,
+                          int64_t P, const uint32_t *counts, const int32_t *row_pair, double *dstar, uint8_t *nan_rep);
 
 // ---- pedigree lists (abfit_inputs.cu) ---------------------------------------------------
 struct ListNode {

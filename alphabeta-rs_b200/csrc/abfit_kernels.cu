@@ -140,8 +140,25 @@ k_select(DevicePools P, int p_base, int n_starts, const abfit_fit *__restrict__ 
 //   D*_i = pred_i + resid[idx_i]      (src/boot_model.rs:50-57)
 // The column is built cooperatively by the warp into a [n_pairs][32] scratch tile
 // (coalesced on the lane axis), then read once per evaluation.
+// DGIVEN (site-block bootstrap): `pred` is the materialised D* matrix [pair_off * n_boot + b * n_pairs + i] and the
+// tile is a copy of the replicate's row; a replicate with a NaN D* is not fitted (NaN row, ABFIT_FIT_NAN).
 // ---------------------------------------------------------------------------------
-template <bool BIG>
+// the record of a replicate that is not fitted because its D* holds a NaN: seven NaNs, ABFIT_FIT_NAN, no iterations
+__device__ __forceinline__ void store_unfitted_replicate(double *rows_out, abfit_fit *fits_out, size_t o, int start_id)
+{
+    double *row = rows_out + o * 7;
+    for (int q = 0; q < 7; ++q) row[q] = nan("");
+    if (!fits_out) return;
+    abfit_fit r;
+    r.theta[0] = r.theta[1] = r.theta[2] = r.theta[3] = nan("");
+    r.cost = r.lse = nan("");
+    r.iters = r.evals = 0;
+    r.status = ABFIT_FIT_NAN;
+    r.start_id = start_id;
+    store_fit(fits_out + o, r);
+}
+
+template <bool BIG, bool DGIVEN = false>
 __global__ void __launch_bounds__(32)
 k_fit_boot(DevicePools P, const WorkItem *__restrict__ items, int n_boot, const abfit_fit *__restrict__ best,
            const double *__restrict__ pred, const double *__restrict__ resid,
@@ -180,10 +197,22 @@ k_fit_boot(DevicePools P, const WorkItem *__restrict__ items, int n_boot, const 
             const bool take = need && idx < end;
             // cooperative build of the D* column of every lane that takes a replicate
             unsigned tm = __ballot_sync(FULL, take);
+            bool nan_rep = false;
             while (tm) {
                 const int tl = __ffs(tm) - 1;
                 tm &= tm - 1;
                 const int b = __shfl_sync(FULL, idx, tl);
+                if (DGIVEN) {
+                    const double *row = pred + (size_t)pb.pair_off * n_boot + (size_t)b * pb.n_pairs;
+                    bool bad = false;
+                    for (int i = lane; i < pb.n_pairs; i += 32) {
+                        const double v = row[i];
+                        bad |= v != v;
+                        tile[(size_t)i * 32 + tl] = v;
+                    }
+                    if (__any_sync(FULL, bad) && lane == tl) nan_rep = true;
+                    continue;
+                }
                 const int32_t *ib = idxp + (size_t)b * pb.n_pairs;
                 for (int i = lane; i < pb.n_pairs; i += 32) {
                     uint32_t ix = (uint32_t)ib[i];
@@ -195,7 +224,9 @@ k_fit_boot(DevicePools P, const WorkItem *__restrict__ items, int n_boot, const 
                 }
             }
             __syncwarp();
-            if (take) {
+            if (DGIVEN && take && nan_rep) {
+                store_unfitted_replicate(rows_out, fits_out, (size_t)it.prob * n_boot + idx, idx);
+            } else if (take) {
                 // simplex = [best, vary x 4]  (src/boot_model.rs:69-75)
                 const double *vv = vary + ((size_t)it.prob * n_boot + idx) * 16;
 #pragma unroll
@@ -208,7 +239,10 @@ k_fit_boot(DevicePools P, const WorkItem *__restrict__ items, int n_boot, const 
         }
         const bool active = (L.phase != PH_IDLE);
         const unsigned amask = __ballot_sync(FULL, active);
-        if (!amask) break;
+        if (!amask) {
+            if (DGIVEN && next < end) continue;  // every lane that took a replicate drew a NaN one
+            break;
+        }
         if (active) {
             const double f =
                 objective(c, Dat, lane, L.xt[0], L.xt[1], L.xt[2], L.xt[3], L.phase != PH_LSE);
@@ -290,7 +324,9 @@ __global__ void k_wide_stats(DevicePools P, const long long *__restrict__ ss_off
     }
 }
 
-template <bool BOOT>
+// DGIVEN (site-block bootstrap, BOOT only): B.pred is the materialised D* matrix [pair_off * n_boot + f * n_pairs + i]
+// and c.D points at the replicate's row; a replicate with a NaN D* is not fitted (NaN row, ABFIT_FIT_NAN).
+template <bool BOOT, bool DGIVEN = false>
 __global__ void __launch_bounds__(32)
 k_fit_wide(DevicePools P, const WorkItem *__restrict__ items, const double *__restrict__ simplices, int n_per_prob,
            NMParams nm, abfit_fit *__restrict__ fits_out, unsigned long long *__restrict__ evals_per_prob, WideBoot B,
@@ -329,7 +365,21 @@ k_fit_wide(DevicePools P, const WorkItem *__restrict__ items, const double *__re
     unsigned long long my_evals = 0;
 
     for (int f = it.first; f < it.first + it.count; ++f) {
-        if (BOOT) {
+        if (DGIVEN) {
+            c.D = B.pred + (size_t)pb.pair_off * n_per_prob + (size_t)f * pb.n_pairs;
+            bool bad = false;
+            for (int i = lane; i < pb.n_pairs; i += 32) bad |= c.D[i] != c.D[i];
+            if (__any_sync(FULL, bad)) {
+                if (lane == 0) store_unfitted_replicate(B.rows_out, fits_out, (size_t)it.prob * n_per_prob + f, f);
+                continue;
+            }
+            const abfit_fit bm = B.best[it.prob];
+            const double *vv = B.vary + ((size_t)it.prob * n_per_prob + f) * 16;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) S.X[q * 32] = bm.theta[q];
+#pragma unroll
+            for (int q = 0; q < 16; ++q) S.X[(4 + q) * 32] = vv[q];
+        } else if (BOOT) {
             const int32_t *ib = B.resample_idx + (size_t)pb.pair_off * n_per_prob + (size_t)f * pb.n_pairs;
             const double *predp = B.pred + pb.pair_off, *residp = B.resid + pb.pair_off;
             for (int i = lane; i < pb.n_pairs; i += 32) {
@@ -724,6 +774,45 @@ int launch_fit_boot_wide(cudaStream_t st, const DevicePools &P, const WorkItem *
         fprintf(stderr, "[abfit] k_fit_wide<boot>: %d blocks x 1 warp, %zu B smem/block\n", n_items, smem_bytes);
     WideBoot B{best, pred, resid, resample_idx, vary, dstar_scratch, (long long)scratch_stride, rows_out, err_flag};
     k_fit_wide<true><<<n_items, 32, smem_bytes, st>>>(P, items, nullptr, n_boot, nm, fits_out, evals_per_prob, B, nullptr, nullptr);
+    ABFIT_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_fit_boot_given(cudaStream_t st, const DevicePools &P, const WorkItem *items, int n_items, int n_boot,
+                          const abfit_fit *best, const double *dstar, const double *vary, double *tile_scratch,
+                          int64_t scratch_stride, NMParams nm, double *rows_out, abfit_fit *fits_out,
+                          unsigned long long *evals_per_prob, size_t smem_bytes, const BigScratch &big)
+{
+    if (n_items <= 0) return 0;
+    if (getenv("ABFIT_DEV_VERBOSE"))
+        fprintf(stderr, "[abfit] k_fit_boot<BIG=%d,DGIVEN=1>: %d blocks x 1 warp, %zu B smem/block\n", big.lm ? 1 : 0,
+                n_items, smem_bytes);
+    if (big.lm) {
+        if (int rc = prep_kernel(k_fit_boot<true, true>, smem_bytes)) return rc;
+        k_fit_boot<true, true><<<n_items, 32, smem_bytes, st>>>(P, items, n_boot, best, dstar, nullptr, nullptr, vary,
+                                                                tile_scratch, (long long)scratch_stride, nm, rows_out,
+                                                                fits_out, evals_per_prob, nullptr, big.x, big.lm, big.lm_stride);
+    } else {
+        if (int rc = prep_kernel(k_fit_boot<false, true>, smem_bytes)) return rc;
+        k_fit_boot<false, true><<<n_items, 32, smem_bytes, st>>>(P, items, n_boot, best, dstar, nullptr, nullptr, vary,
+                                                                 tile_scratch, (long long)scratch_stride, nm, rows_out,
+                                                                 fits_out, evals_per_prob, nullptr, nullptr, nullptr, 0);
+    }
+    ABFIT_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int launch_fit_boot_wide_given(cudaStream_t st, const DevicePools &P, const WorkItem *items, int n_items, int n_boot,
+                               const abfit_fit *best, const double *dstar, const double *vary, NMParams nm,
+                               double *rows_out, abfit_fit *fits_out, unsigned long long *evals_per_prob, size_t smem_bytes)
+{
+    if (n_items <= 0) return 0;
+    if (int rc = prep_kernel(k_fit_wide<true, true>, smem_bytes, false)) return rc;
+    if (getenv("ABFIT_DEV_VERBOSE"))
+        fprintf(stderr, "[abfit] k_fit_wide<boot,DGIVEN=1>: %d blocks x 1 warp, %zu B smem/block\n", n_items, smem_bytes);
+    WideBoot B{best, dstar, nullptr, nullptr, vary, nullptr, 0, rows_out, nullptr};
+    k_fit_wide<true, true><<<n_items, 32, smem_bytes, st>>>(P, items, nullptr, n_boot, nm, fits_out, evals_per_prob, B, nullptr,
+                                                            nullptr);
     ABFIT_CUDA(cudaGetLastError());
     return 0;
 }

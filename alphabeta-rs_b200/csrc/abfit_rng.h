@@ -46,4 +46,13 @@ ABFIT_HD inline double vary_coordinate(uint64_t seed, uint64_t problem_id, uint6
     return uniform(lo, hi, u01(seed, 2, problem_id, b, (uint64_t)(v * 4 + j)));
 }
 
+// site-block bootstrap: draw d of replicate b picks one of the window's n_blocks blocks (stream 5; streams 1-3 are
+// starts, vary vertices and resamples, 4 the simulator)
+ABFIT_HD inline int32_t site_boot_block(uint64_t seed, uint64_t problem_id, uint64_t b, uint64_t d, int32_t n_blocks)
+{
+    int32_t k = (int32_t)(u01(seed, 5, problem_id, b, d) * (double)n_blocks);
+    if (k >= n_blocks) k = n_blocks - 1;
+    return k;
+}
+
 }  // namespace abfit

@@ -247,6 +247,47 @@ int abfit_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const doubl
                             double thr, double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out,
                             double *methsum_out, int64_t *nvalid_out, float kernel_ms[2], int32_t *launches_out);
 
+/* ---- site-block bootstrap ----------------------------------------------------
+ * An opt-in alternative to abfit_boot_batch's residual bootstrap: instead of resampling pair residuals, every
+ * replicate resamples the window's SITES in blocks and recomputes the observed divergence exactly.  Window p
+ * (sites [seg_offsets[p], seg_offsets[p+1]), problem p) is cut into B_p = ceil(L_p / block_sites) blocks of
+ * consecutive sites from its first site (the last block holds the remainder); replicate b draws B_p blocks with
+ * replacement, draw d picking block (int)(u01(seed, 5, key, b, d) * B_p) (clamped to B_p - 1), key = problem_ids[p]
+ * when given, else first_problem_id + p.  abfit_gen_site_boot_counts gives the multiplicities on the host.
+ * A replicate's pair sums are integer combinations of the per-block sums of abfit_divergence, so
+ * D*[b][row] = (double)sum diff / (2.0 * (double)sum cnt) is exact.  A replicate in which a pedigree row's pair has
+ * no valid site (sum cnt = 0, D* = NaN) is not fitted: its row is seven NaNs, its fit status ABFIT_FIT_NAN (iters 0),
+ * and it is counted in nan_reps_out.  Every other replicate is refitted like abfit_boot_batch's, from the simplex
+ * [best, vary x 4] with vary = abfit_gen_vary_vertices(seed, key, n_boot, best[p].theta); p0uu, eqp and eqp_weight
+ * stay each problem's values.
+ *  probs         [n_probs] the observed problems (the fit's); pedigree rows pair with `pairs`
+ *  pairs         [sum n_pairs][2] samples (i, j), i != j < S, of every pedigree row (abfit_pedigree_graph /
+ *                abfit_sim_tree_pairs columns 0 and 1)
+ *  status, posterior_max, meth_lvl, S, L, thr   as in abfit_divergence (host arrays; device arrays for _device)
+ *  seg_offsets   [n_probs + 1] host array, window p = problem p; every window holds at least one site
+ *  block_sites   >= 1, < 2^31
+ *  best          [n_probs] from abfit_fit_batch
+ *  rows_out      [n_probs][n_boot][7], fits_out [n_probs][n_boot] (may be NULL), analysis_out [n_probs][32]
+ *                (abfit_analyze of every window's rows; may be NULL), dstar_out [sum n_boot * n_pairs] in the
+ *                layout of abfit_boot_batch's resample_idx (may be NULL), nan_reps_out [n_probs] (may be NULL)
+ * Refused before any launch: block_sites < 1, an empty window, bad pairs (ABFIT_ERR_ARG); per-block partial sums
+ * that do not fit in free device memory (ABFIT_ERR_TOO_LARGE). */
+void abfit_gen_site_boot_counts(uint64_t seed, uint64_t problem_key, int32_t n_boot, int32_t n_blocks,
+                                uint32_t *counts_out /* [n_boot][n_blocks] */);
+int abfit_site_boot_batch(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_probs, const int32_t *pairs,
+                          const uint8_t *status, const double *posterior_max, const double *meth_lvl, int32_t S, int64_t L,
+                          const int64_t *seg_offsets, double thr, int64_t block_sites, const abfit_fit *best,
+                          int32_t n_boot, uint64_t seed, uint64_t first_problem_id, const uint64_t *problem_ids,
+                          int32_t max_iters, double sd_tol, uint32_t flags, double *rows_out, abfit_fit *fits_out,
+                          double *analysis_out, double *dstar_out, int32_t *nan_reps_out);
+int abfit_site_boot_batch_device(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_probs, const int32_t *pairs,
+                                 const uint8_t *d_status, const double *d_posterior_max, const double *d_meth_lvl, int32_t S,
+                                 int64_t L, const int64_t *seg_offsets, double thr, int64_t block_sites,
+                                 const abfit_fit *best, int32_t n_boot, uint64_t seed, uint64_t first_problem_id,
+                                 const uint64_t *problem_ids, int32_t max_iters, double sd_tol, uint32_t flags,
+                                 double *rows_out, abfit_fit *fits_out, double *analysis_out, double *dstar_out,
+                                 int32_t *nan_reps_out);
+
 /* ---- staged, device-resident interface ------------------------------------
  * Same computation as abfit_fit_batch + abfit_boot_batch, split into upload /
  * run / download so a caller (bench.py, the metaprofile driver) can keep inputs

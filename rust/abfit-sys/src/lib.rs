@@ -123,6 +123,24 @@ extern "C" {
         resid: *const f64, n_boot: i32, resample_idx: *const i32, vary_vertices: *const f64, max_iters: i32, sd_tol: f64,
         flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit,
     ) -> c_int;
+    /// site-block bootstrap: multiplicities [n_boot][n_blocks] of a window's blocks (generator stream 5)
+    pub fn abfit_gen_site_boot_counts(seed: u64, problem_key: u64, n_boot: i32, n_blocks: i32, counts_out: *mut u32);
+    /// site-block bootstrap of fitted windows: exact D* from resampled blocks of sites, refitted like `boot_model::run`
+    pub fn abfit_site_boot_batch(
+        ctx: *mut abfit_ctx, probs: *const abfit_problem, n_probs: i32, pairs: *const i32, status: *const u8,
+        posterior_max: *const f64, meth_lvl: *const f64, s: i32, l: i64, seg_offsets: *const i64, thr: f64,
+        block_sites: i64, best: *const abfit_fit, n_boot: i32, seed: u64, first_problem_id: u64, problem_ids: *const u64,
+        max_iters: i32, sd_tol: f64, flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit, analysis_out: *mut f64,
+        dstar_out: *mut f64, nan_reps_out: *mut i32,
+    ) -> c_int;
+    /// the same with the three site arrays in device memory
+    pub fn abfit_site_boot_batch_device(
+        ctx: *mut abfit_ctx, probs: *const abfit_problem, n_probs: i32, pairs: *const i32, d_status: *const u8,
+        d_posterior_max: *const f64, d_meth_lvl: *const f64, s: i32, l: i64, seg_offsets: *const i64, thr: f64,
+        block_sites: i64, best: *const abfit_fit, n_boot: i32, seed: u64, first_problem_id: u64, problem_ids: *const u64,
+        max_iters: i32, sd_tol: f64, flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit, analysis_out: *mut f64,
+        dstar_out: *mut f64, nan_reps_out: *mut i32,
+    ) -> c_int;
     /// `alphabeta::run` (src/alphabeta.rs:23-59) for every window of a metaprofile (src/cli/metaprofile.rs:50-72)
     pub fn abfit_alphabeta_batch(
         ctx: *mut abfit_ctx, probs: *const abfit_problem, n_probs: i32, n_starts: i32, simplices: *const f64, n_boot: i32,
