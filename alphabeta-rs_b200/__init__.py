@@ -151,6 +151,11 @@ def _load() -> C.CDLL:
         "abfit_sim_equilibrium": (C.c_int, [dbl, dbl, C.POINTER(dbl), C.POINTER(dbl)]),
         "abfit_simulate": (C.c_int, [vp, vp, vp, i64, i64, vp, vp, vp]),
         "abfit_simulate_device": (C.c_int, [vp, vp, vp, i64, i64, vp, vp, vp, C.POINTER(C.c_float)]),
+        "abfit_parse_region_line": (C.c_int, [C.c_char_p, C.POINTER(i32), C.POINTER(i64), C.POINTER(i64)]),
+        "abfit_region_ranges": (C.c_int, [vp, i64, vp, vp, vp, i32, vp, vp]),
+        "abfit_region_divergence": (C.c_int, [vp, vp, vp, vp, i32, i64, vp, vp, i32, dbl, vp, vp, vp, vp, vp, vp]),
+        "abfit_region_divergence_device": (C.c_int, [vp, vp, vp, vp, i32, i64, vp, vp, i32, dbl, vp, vp, vp, vp, vp, vp,
+                                                     C.POINTER(C.c_float), C.POINTER(i32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
@@ -174,7 +179,8 @@ EXPORTED_SYMBOLS = (
     "abfit_write_npy_f64 abfit_write_metaprofile_results abfit_plot_metaplot abfit_plot_bootstrap "
     "abfit_sim_tree_build abfit_sim_tree_from_arrays abfit_sim_tree_info abfit_sim_tree_pairs abfit_sim_tree_thresholds "
     "abfit_sim_tree_free abfit_sim_equilibrium abfit_simulate abfit_simulate_device "
-    "abfit_gen_site_boot_counts abfit_site_boot_batch abfit_site_boot_batch_device"
+    "abfit_gen_site_boot_counts abfit_site_boot_batch abfit_site_boot_batch_device "
+    "abfit_parse_region_line abfit_region_ranges abfit_region_divergence abfit_region_divergence_device"
 ).split()
 
 
@@ -593,6 +599,41 @@ class Context:
                                (C.c_void_p(d_status), C.c_void_p(d_post), C.c_void_p(d_meth)), S, L, seg_offsets, best,
                                n_boot, seed, block_sites, thr, first_problem_id, problem_ids, max_iters, sd_tol, flags)
 
+    # -- genomic regions (include/abfit.h, abfit_region_divergence) -------------------------------
+    def _region_div(self, fn, inputs, S, L, lo, hi, thr, extra=()):
+        lo = np.ascontiguousarray(lo, dtype=np.int64).reshape(-1)
+        hi = np.ascontiguousarray(hi, dtype=np.int64).reshape(-1)
+        if lo.shape != hi.shape:
+            raise ValueError(f"lo has {lo.size} entries, hi {hi.size}")
+        W, P = lo.size, S * (S - 1) // 2
+        D = np.empty((W, P))
+        diff = np.empty((W, P), dtype=np.uint64)
+        cnt = np.empty((W, P), dtype=np.uint64)
+        p0uu = np.empty(W)
+        methsum = np.empty((W, S))
+        nvalid = np.empty((W, S), dtype=np.int64)
+        _check(fn(self._h, *inputs, S, L, _ptr(lo), _ptr(hi), W, thr, _ptr(D), _ptr(diff), _ptr(cnt), _ptr(p0uu),
+                  _ptr(methsum), _ptr(nvalid), *extra))
+        return {"D": D, "diff": diff, "cnt": cnt, "p0uu": p0uu, "methsum": methsum, "nvalid": nvalid}
+
+    def region_divergence(self, status, posterior_max, meth_lvl, lo, hi, thr=0.99):
+        """Observed divergence of the regions [lo[w], hi[w]) of the [S, L] site arrays (abfit_region_divergence): every
+        output of region w equals dmatrix(..., seg_offsets=[lo[w], hi[w]]) bit for bit.  -> the dmatrix() dict"""
+        status = np.ascontiguousarray(status, dtype=np.uint8)
+        S, L = status.shape
+        post, meth = _f64(posterior_max, (S, L)), _f64(meth_lvl, (S, L))
+        return self._region_div(_lib.abfit_region_divergence, (_ptr(status), _ptr(post), _ptr(meth)), S, L, lo, hi, thr)
+
+    def region_divergence_device(self, d_status: int, d_post: int, d_meth: int, S: int, L: int, lo, hi, thr=0.99):
+        """region_divergence() with the three [S, L] site arrays in device memory (ints: device pointers; the stream that
+        wrote them must be synchronised); adds kernel_ms (device time of the call) and launches"""
+        ms, launches = C.c_float(), C.c_int32()
+        out = self._region_div(_lib.abfit_region_divergence_device,
+                               (C.c_void_p(d_status), C.c_void_p(d_post), C.c_void_p(d_meth)), S, L, lo, hi, thr,
+                               (C.byref(ms), C.byref(launches)))
+        out["kernel_ms"], out["launches"] = ms.value, launches.value
+        return out
+
     def batch(self, probs: Sequence[Problem]) -> "Batch":
         return Batch(self, probs)
 
@@ -920,6 +961,32 @@ def parse_methylome_buffer(data: bytes, invert_strand: bool = False, skip_first_
     if want_lines:
         out["line_off"], out["line_len"] = off[:k], ln[:k]
     return out
+
+
+def parse_region_line(line: str):
+    """abfit_parse_region_line: one BED line -> (chromosome, start0, end), None for a line that is not a region (empty,
+    '#', track, browser); AbfitError for a malformed line"""
+    c, a, b = C.c_int32(), C.c_int64(), C.c_int64()
+    rc = _lib.abfit_parse_region_line(line.encode(), C.byref(c), C.byref(a), C.byref(b))
+    if rc == 1:
+        return None
+    _check(rc)
+    return c.value, a.value, b.value
+
+
+def region_ranges(sites, chrom, start0, end):
+    """abfit_region_ranges: regions (chromosome, 0-based start, end) -> site index ranges (lo, hi) of `sites`
+    (SITE_DTYPE, grouped by chromosome, positions non-decreasing within each)"""
+    sites = np.ascontiguousarray(sites, dtype=SITE_DTYPE)
+    chrom = np.ascontiguousarray(chrom, dtype=np.int32).reshape(-1)
+    start0 = np.ascontiguousarray(start0, dtype=np.int64).reshape(-1)
+    end = np.ascontiguousarray(end, dtype=np.int64).reshape(-1)
+    if not (chrom.shape == start0.shape == end.shape):
+        raise ValueError(f"chrom, start0 and end have {chrom.size}, {start0.size} and {end.size} entries")
+    lo, hi = np.empty(chrom.size, dtype=np.int64), np.empty(chrom.size, dtype=np.int64)
+    _check(_lib.abfit_region_ranges(_ptr(sites), len(sites), _ptr(chrom), _ptr(start0), _ptr(end), chrom.size, _ptr(lo),
+                                    _ptr(hi)))
+    return lo, hi
 
 
 def build_pedigree(ctx: Context, nodelist: str, edgelist: str, posterior_max_filter: float = 0.99):

@@ -1518,6 +1518,115 @@ int abfit_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const doubl
 }
 
 // ---------------------------------------------------------------------------------------
+// per-region divergence (abfit_regions.cu): every region = the single window {lo, hi} of abfit_divergence
+// ---------------------------------------------------------------------------------------
+static int region_divergence_impl(abfit_ctx *ctx, bool device_inputs, const uint8_t *status, const double *posterior_max,
+                                  const double *meth_lvl, int32_t S, int64_t L, const int64_t *lo, const int64_t *hi, int32_t W,
+                                  double thr, double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out,
+                                  double *methsum_out, int64_t *nvalid_out, float *ms_out, int32_t *launches_out)
+{
+    // every refusal that needs no device comes first
+    if (!ctx || !status || !posterior_max || !meth_lvl || S <= 0 || S > 65535 || L < 0 || !lo || !hi || W <= 0) {
+        set_error("region divergence: missing or out-of-range argument");
+        return ABFIT_ERR_ARG;
+    }
+    for (int32_t w = 0; w < W; ++w)
+        if (lo[w] < 0 || lo[w] > hi[w] || hi[w] > L) {
+            set_error("region divergence: region " + std::to_string(w) + " [" + std::to_string(lo[w]) + ", " +
+                      std::to_string(hi[w]) + ") is not a site range of [0, " + std::to_string(L) + ")");
+            return ABFIT_ERR_ARG;
+        }
+    RegionPlan plan;
+    if (int rc = plan_regions(S, L, lo, hi, W, plan)) return rc;
+    const size_t P = (size_t)S * (S - 1) / 2, n = (size_t)S * (size_t)L;
+    ABFIT_CUDA(cudaSetDevice(ctx->device));
+    {
+        const size_t need = (size_t)W * P * 24 + (size_t)W * S * 16 + (size_t)W * 8 + plan.bytes + (device_inputs ? 0 : n * 17);
+        size_t fr = 0, tot = 0;
+        ABFIT_CUDA(cudaMemGetInfo(&fr, &tot));
+        if (need > fr) {
+            set_error("region divergence: " + std::to_string(W) + " regions x " + std::to_string(P) + " pairs need about " +
+                      std::to_string(need >> 20) + " MiB of device memory, " + std::to_string(fr >> 20) + " MiB are free");
+            return ABFIT_ERR_TOO_LARGE;
+        }
+    }
+    cudaStream_t st = ctx->stream;
+    DevBuf<uint8_t> d_status;
+    DevBuf<double> d_post, d_meth, d_D, d_methsum, d_p0uu;
+    DevBuf<unsigned long long> d_diff, d_cnt;
+    DevBuf<long long> d_nvalid;
+    if (!device_inputs) {
+        if (int rc = d_status.ensure(n)) return rc;
+        if (int rc = d_post.ensure(n)) return rc;
+        if (int rc = d_meth.ensure(n)) return rc;
+        if (n) {
+            ABFIT_CUDA(cudaMemcpyAsync(d_status.p, status, n, cudaMemcpyHostToDevice, st));
+            ABFIT_CUDA(cudaMemcpyAsync(d_post.p, posterior_max, n * 8, cudaMemcpyHostToDevice, st));
+            ABFIT_CUDA(cudaMemcpyAsync(d_meth.p, meth_lvl, n * 8, cudaMemcpyHostToDevice, st));
+        }
+        status = d_status.p;
+        posterior_max = d_post.p;
+        meth_lvl = d_meth.p;
+    }
+    if (int rc = d_D.ensure((size_t)W * P)) return rc;
+    if (int rc = d_diff.ensure((size_t)W * P)) return rc;
+    if (int rc = d_cnt.ensure((size_t)W * P)) return rc;
+    if (int rc = d_methsum.ensure((size_t)W * S)) return rc;
+    if (int rc = d_nvalid.ensure((size_t)W * S)) return rc;
+    if (int rc = d_p0uu.ensure(W)) return rc;
+    struct Events {  // destroyed on every way out
+        cudaEvent_t e[2] = {nullptr, nullptr};
+        ~Events()
+        {
+            for (auto &x : e)
+                if (x) cudaEventDestroy(x);
+        }
+    } ev;
+    if (ms_out) {
+        ABFIT_CUDA(cudaEventCreate(&ev.e[0]));
+        ABFIT_CUDA(cudaEventCreate(&ev.e[1]));
+        ABFIT_CUDA(cudaEventRecord(ev.e[0], st));
+    }
+    int launches = 0;
+    if (int rc = run_region_divergence(st, &ctx->div_arena, plan, status, posterior_max, meth_lvl, S, L, lo, hi, W, thr, d_D.p,
+                                       d_diff.p, d_cnt.p, d_methsum.p, d_nvalid.p, d_p0uu.p, &launches))
+        return rc;
+    if (ms_out) {
+        ABFIT_CUDA(cudaEventRecord(ev.e[1], st));
+        ABFIT_CUDA(cudaEventSynchronize(ev.e[1]));
+        ABFIT_CUDA(cudaEventElapsedTime(ms_out, ev.e[0], ev.e[1]));
+    }
+    if (launches_out) *launches_out = launches;
+    if (D_out && P) ABFIT_CUDA(cudaMemcpyAsync(D_out, d_D.p, (size_t)W * P * 8, cudaMemcpyDeviceToHost, st));
+    if (diff_out && P) ABFIT_CUDA(cudaMemcpyAsync(diff_out, d_diff.p, (size_t)W * P * 8, cudaMemcpyDeviceToHost, st));
+    if (cnt_out && P) ABFIT_CUDA(cudaMemcpyAsync(cnt_out, d_cnt.p, (size_t)W * P * 8, cudaMemcpyDeviceToHost, st));
+    if (p0uu_out) ABFIT_CUDA(cudaMemcpyAsync(p0uu_out, d_p0uu.p, (size_t)W * 8, cudaMemcpyDeviceToHost, st));
+    if (methsum_out) ABFIT_CUDA(cudaMemcpyAsync(methsum_out, d_methsum.p, (size_t)W * S * 8, cudaMemcpyDeviceToHost, st));
+    if (nvalid_out) ABFIT_CUDA(cudaMemcpyAsync(nvalid_out, d_nvalid.p, (size_t)W * S * 8, cudaMemcpyDeviceToHost, st));
+    ABFIT_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int abfit_region_divergence(abfit_ctx *ctx, const uint8_t *status, const double *posterior_max, const double *meth_lvl,
+                            int32_t S, int64_t L, const int64_t *region_lo, const int64_t *region_hi, int32_t W, double thr,
+                            double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out, double *methsum_out,
+                            int64_t *nvalid_out)
+{
+    return region_divergence_impl(ctx, false, status, posterior_max, meth_lvl, S, L, region_lo, region_hi, W, thr, D_out,
+                                  diff_out, cnt_out, p0uu_out, methsum_out, nvalid_out, nullptr, nullptr);
+}
+
+int abfit_region_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const double *d_posterior_max,
+                                   const double *d_meth_lvl, int32_t S, int64_t L, const int64_t *region_lo,
+                                   const int64_t *region_hi, int32_t W, double thr, double *D_out, uint64_t *diff_out,
+                                   uint64_t *cnt_out, double *p0uu_out, double *methsum_out, int64_t *nvalid_out,
+                                   float *kernel_ms, int32_t *launches_out)
+{
+    return region_divergence_impl(ctx, true, d_status, d_posterior_max, d_meth_lvl, S, L, region_lo, region_hi, W, thr, D_out,
+                                  diff_out, cnt_out, p0uu_out, methsum_out, nvalid_out, kernel_ms, launches_out);
+}
+
+// ---------------------------------------------------------------------------------------
 // site-block bootstrap: per-block partial sums (the observed-divergence path over a list of block windows) -> D* of
 // every replicate (k_siteboot_dstar) -> the bootstrap refit kernels on the given D* (DGIVEN instantiations)
 // ---------------------------------------------------------------------------------------

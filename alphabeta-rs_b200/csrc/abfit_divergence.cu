@@ -19,7 +19,7 @@
 namespace abfit {
 
 constexpr int SB_WORDS = 64;           // words (64 sites) per super-block = one warp's share in k_pack
-constexpr int64_t EXACT_MAX = 65536;   // windows up to this many sites: sequential (bit-exact) methsum
+constexpr int64_t EXACT_MAX = DIV_EXACT_MAX;   // windows up to this many sites: sequential (bit-exact) methsum
 constexpr int FIN_WARPS = 4;           // warps per block of the per-sample finalisation kernels
 
 struct SuperBlock {

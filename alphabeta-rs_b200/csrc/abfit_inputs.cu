@@ -250,6 +250,9 @@ struct PedGraph {
 
 }  // namespace
 
+bool abfit::parse_chromosome_name(std::string_view s, int32_t &c) { return parse_chromosome(s, c); }
+bool abfit::parse_u32_field(std::string_view s, uint32_t &v) { return parse_u32(s, v); }
+
 // nodes: split on \n and \r, skip the header, id = index after the header (src/pedigree.rs:99-116); edges: the first
 // two fields of every line after the header (src/pedigree.rs:123-135), names not yet resolved
 int abfit::read_node_edge_lists(const char *nodelist_path, const char *edgelist_path, std::vector<ListNode> &nodes,

@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <string>
+#include <string_view>
 #include <vector>
 
 #include "abfit_nm.cuh"
@@ -115,6 +116,8 @@ int run_divergence(cudaStream_t st, const uint8_t *d_status, const double *d_pos
 // two-pass path sum meth_lvl in different trees, so a call that is split over devices decides this once, for all of
 // its windows, and passes the answer to every shard: each window then gets the bits one device gives it.
 bool div_long_windows(const int64_t *h_seg, int W);
+// windows of at most this many sites sum meth_lvl sequentially in site order (bit-identical to the reference)
+constexpr int64_t DIV_EXACT_MAX = 65536;
 
 // ---- site-block bootstrap (abfit_siteboot.cu) ---------------------------------------------
 constexpr int SB_THREADS = 128;  // pedigree rows per block of k_siteboot_dstar
@@ -135,7 +138,32 @@ int launch_siteboot_counts(cudaStream_t st, uint64_t seed, uint64_t first_proble
 int launch_siteboot_dstar(cudaStream_t st, const SiteBootItem *items, int n_items, int n_boot, const uint2 *partials,
                           int64_t P, const uint32_t *counts, const int32_t *row_pair, double *dstar, uint8_t *nan_rep);
 
+// ---- per-region divergence (abfit_regions.cu) ---------------------------------------------
+// Regions of at most DIV_EXACT_MAX sites get their diff / cnt from prefix sums over the pieces between region endpoints
+// and their methsum from a sequential pass; longer ones run through run_divergence alone (its long-window tree).
+struct RegionEdge {
+    int32_t region, lo_row, hi_row, pad;  // rows of this chunk's prefix sums to subtract / add (-1: in another chunk)
+};
+struct RegionPlan {
+    std::vector<int64_t> cuts;                    // sorted, unique endpoints of the non-empty short regions
+    std::vector<int32_t> longs;                   // regions of more than DIV_EXACT_MAX sites
+    std::vector<std::vector<RegionEdge>> edges;   // per chunk of pieces
+    int64_t chunk = 1;                            // pieces per run_divergence call
+    size_t max_edges = 0;
+    size_t bytes = 0;                             // device scratch of the call (outputs and inputs not included)
+};
+// lo / hi: host arrays [W], already checked to be ranges of [0, L]
+int plan_regions(int S, int64_t L, const int64_t *lo, const int64_t *hi, int W, RegionPlan &plan);
+// every pointer but h_lo / h_hi is device memory; outputs [W][P] / [W][S] / [W]
+int run_region_divergence(cudaStream_t st, DivArena *arena, const RegionPlan &plan, const uint8_t *d_status,
+                          const double *d_post, const double *d_meth, int S, int64_t L, const int64_t *h_lo,
+                          const int64_t *h_hi, int W, double thr, double *d_D, unsigned long long *d_diff,
+                          unsigned long long *d_cnt, double *d_methsum, long long *d_nvalid, double *d_p0uu, int *launches);
+
 // ---- pedigree lists (abfit_inputs.cu) ---------------------------------------------------
+// the methylome parser's chromosome rule (Numbered(n) -> n, M -> 256, C -> 257, "chr" prefixes dropped) and its u32
+bool parse_chromosome_name(std::string_view s, int32_t &c);
+bool parse_u32_field(std::string_view s, uint32_t &v);
 struct ListNode {
     size_t id;  // line index after the header
     std::string file, name;

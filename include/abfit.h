@@ -369,6 +369,43 @@ int abfit_place_sites(const abfit_gene *genes, int32_t n_genes, const abfit_cg_s
                       const abfit_window_args *args, int32_t *distribution_out, int64_t *n_assign_out,
                       int64_t assign_cap, int64_t *assign_site, int32_t *assign_window);
 
+/* ---- arbitrary genomic regions (BED files) --------------------------------------------
+ * abfit_parse_region_line: one BED line -> chromosome, start0, end.  0 = parsed; 1 = not a region (empty line, '#',
+ * `track` or `browser`); < 0 = malformed (fewer than three columns, a chromosome or an integer that does not parse,
+ * end < start0; abfit_last_error says which).  Columns are separated by blanks or tabs; only the first three are read
+ * (column 4, when present, is the region's name to callers).  The chromosome column follows the methylome parser's rule
+ * (abfit_parse_methylome_line): Numbered(n) -> n, M -> 256, C -> 257, "chr" prefixes dropped, so a BED file names
+ * chromosomes as the methylome files do.  Coordinates are 0-based, half-open: the region covers the 1-based site
+ * positions start0 + 1 .. end (abfit_cg_site.start).  Regions ignore strand: unlike metaprofile's gene windows, which
+ * match a site's strand to its gene's, a region holds the sites of both strands. */
+int abfit_parse_region_line(const char *line, int32_t *chrom_out, int64_t *start0_out, int64_t *end_out);
+/* W regions -> site index ranges [lo_out[w], hi_out[w]) of `sites` by binary search (host only, multi-threaded for large
+ * W).  Refused (ABFIT_ERR_ARG, the message names the chromosome and the site index): a chromosome whose sites do not form
+ * one contiguous run, positions that decrease within a chromosome, a region with end < start0.  A region on a chromosome
+ * without sites gets the empty range [0, 0). */
+int abfit_region_ranges(const abfit_cg_site *sites, int64_t n_sites, const int32_t *chrom, const int64_t *start0,
+                        const int64_t *end, int32_t W, int64_t *lo_out, int64_t *hi_out);
+/* Observed divergence of W regions = site ranges [region_lo[w], region_hi[w]) of the [S][L] site arrays (host arrays;
+ * device arrays for _device).  Regions may overlap, nest, repeat, come in any order or be empty.  Every output of region w
+ * equals, bit for bit, what abfit_divergence returns for the single window seg = {region_lo[w], region_hi[w]} of the same
+ * arrays; an empty region gets what an empty window gets: D = NaN, diff = cnt = 0, methsum = 0, nvalid = 0, p0uu = NaN.
+ * No site is copied: diff / cnt of regions of at most 65536 sites are differences of exact u64 prefix sums over the
+ * pieces between region endpoints, their methsum the sequential sum; longer regions run as single windows.
+ *  outputs as abfit_divergence's with W windows (each may be NULL)
+ *  kernel_ms  (_device, may be NULL): device time of the call's work on the context stream; launches_out: kernels launched
+ * The _device twin follows abfit_divergence_device's stream rule (inputs complete before the call).  Refused before any
+ * launch: a range outside [0, L] or with lo > hi, W <= 0 (ABFIT_ERR_ARG); W x S(S-1)/2 x 24 bytes of outputs plus one
+ * chunk of piece sums that do not fit in free device memory (ABFIT_ERR_TOO_LARGE). */
+int abfit_region_divergence(abfit_ctx *ctx, const uint8_t *status, const double *posterior_max, const double *meth_lvl,
+                            int32_t S, int64_t L, const int64_t *region_lo, const int64_t *region_hi, int32_t W, double thr,
+                            double *D_out, uint64_t *diff_out, uint64_t *cnt_out, double *p0uu_out, double *methsum_out,
+                            int64_t *nvalid_out);
+int abfit_region_divergence_device(abfit_ctx *ctx, const uint8_t *d_status, const double *d_posterior_max,
+                                   const double *d_meth_lvl, int32_t S, int64_t L, const int64_t *region_lo,
+                                   const int64_t *region_hi, int32_t W, double thr, double *D_out, uint64_t *diff_out,
+                                   uint64_t *cnt_out, double *p0uu_out, double *methsum_out, int64_t *nvalid_out,
+                                   float *kernel_ms, int32_t *launches_out);
+
 /* ---- post-processing ------------------------------------------------------ */
 /* Replaces RawAnalysis::analyze (src/analysis.rs:50-98). rows [n][7] -> out[32]: 8 means,
  * 8 sds (ddof 1), 8 (q0.025, q0.975) pairs, field order alpha, beta, beta/alpha, weight,

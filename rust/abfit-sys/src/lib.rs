@@ -141,6 +141,26 @@ extern "C" {
         max_iters: i32, sd_tol: f64, flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit, analysis_out: *mut f64,
         dstar_out: *mut f64, nan_reps_out: *mut i32,
     ) -> c_int;
+    /// one BED line -> (chromosome, 0-based start, end): 0 parsed, 1 not a region (empty, '#', track, browser), < 0 malformed
+    pub fn abfit_parse_region_line(line: *const c_char, chrom_out: *mut i32, start0_out: *mut i64, end_out: *mut i64) -> c_int;
+    /// regions -> site index ranges [lo, hi) of a site list grouped by chromosome (binary search, host)
+    pub fn abfit_region_ranges(
+        sites: *const abfit_cg_site, n_sites: i64, chrom: *const i32, start0: *const i64, end: *const i64, w: i32,
+        lo_out: *mut i64, hi_out: *mut i64,
+    ) -> c_int;
+    /// observed divergence of every region, each equal bit for bit to `abfit_divergence` on the window {lo, hi}
+    pub fn abfit_region_divergence(
+        ctx: *mut abfit_ctx, status: *const u8, posterior_max: *const f64, meth_lvl: *const f64, s: i32, l: i64,
+        region_lo: *const i64, region_hi: *const i64, w: i32, thr: f64, d_out: *mut f64, diff_out: *mut u64,
+        cnt_out: *mut u64, p0uu_out: *mut f64, methsum_out: *mut f64, nvalid_out: *mut i64,
+    ) -> c_int;
+    /// the same with the three site arrays in device memory
+    pub fn abfit_region_divergence_device(
+        ctx: *mut abfit_ctx, d_status: *const u8, d_posterior_max: *const f64, d_meth_lvl: *const f64, s: i32, l: i64,
+        region_lo: *const i64, region_hi: *const i64, w: i32, thr: f64, d_out: *mut f64, diff_out: *mut u64,
+        cnt_out: *mut u64, p0uu_out: *mut f64, methsum_out: *mut f64, nvalid_out: *mut i64, kernel_ms: *mut f32,
+        launches_out: *mut i32,
+    ) -> c_int;
     /// `alphabeta::run` (src/alphabeta.rs:23-59) for every window of a metaprofile (src/cli/metaprofile.rs:50-72)
     pub fn abfit_alphabeta_batch(
         ctx: *mut abfit_ctx, probs: *const abfit_problem, n_probs: i32, n_starts: i32, simplices: *const f64, n_boot: i32,
