@@ -65,6 +65,7 @@ struct abfit_ctx {
     static constexpr int SX_CHUNKS = 64;
     int *h_sx_counts = nullptr;  // pinned [SX_CHUNKS]
     int *d_sx_ready = nullptr;
+    cudaEvent_t sx_reset = nullptr;  // recorded behind the counter's reset: the watching kernel's stream waits on it
     cudaDeviceProp prop{};
     int smem_optin = 0;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
@@ -276,6 +277,7 @@ void abfit_ctx_destroy(abfit_ctx *ctx)
     if (ctx->pipe_start) cudaEventDestroy(ctx->pipe_start);
     if (ctx->idx_done) cudaEventDestroy(ctx->idx_done);
     if (ctx->copy_done) cudaEventDestroy(ctx->copy_done);
+    if (ctx->sx_reset) cudaEventDestroy(ctx->sx_reset);
     if (ctx->h_sx_counts) cudaFreeHost(ctx->h_sx_counts);
     if (ctx->d_sx_ready) cudaFree(ctx->d_sx_ready);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -1102,9 +1104,11 @@ static int alphabeta_impl(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_
         ABFIT_CUDA(cudaHostAlloc(&ctx->h_sx_counts, abfit_ctx::SX_CHUNKS * sizeof(int), cudaHostAllocDefault));
         ABFIT_CUDA(cudaMalloc(&ctx->d_sx_ready, sizeof(int)));
     }
+    if (!ctx->sx_reset) ABFIT_CUDA(cudaEventCreateWithFlags(&ctx->sx_reset, cudaEventDisableTiming));
     {
         const int per = std::max(256, (n_probs + abfit_ctx::SX_CHUNKS - 1) / abfit_ctx::SX_CHUNKS);  // windows per chunk
         ABFIT_CUDA(cudaMemsetAsync(ctx->d_sx_ready, 0, sizeof(int), ctx->copy_stream));
+        ABFIT_CUDA(cudaEventRecord(ctx->sx_reset, ctx->copy_stream));
         int c = 0;
         for (int p0 = 0; p0 < n_probs; p0 += per, ++c) {
             const int p1 = std::min(n_probs, p0 + per);
@@ -1130,7 +1134,9 @@ static int alphabeta_impl(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_
     phase("plan bootstrap items");
     // the continuous-scheduling kernel watches the upload's counter; every other kernel family waits for the whole copy
     const bool watch_upload = b->jit && b->jit->sched == 2 && !b->shape.wide && !getenv("ABFIT_DEV_NO_UPLOAD_WATCH");
-    if (!watch_upload) ABFIT_CUDA(cudaStreamWaitEvent(st, ctx->copy_done, 0));
+    // watching: the counter still holds the previous call's count until its reset lands, so the kernel waits for that
+    ABFIT_CUDA(cudaStreamWaitEvent(st, watch_upload ? ctx->sx_reset : ctx->copy_done, 0));
+    if (verbose && watch_upload) fprintf(stderr, "[abfit] alphabeta_batch: the multi-start kernel watches the upload\n");
     b->sx_ready = watch_upload ? ctx->d_sx_ready : nullptr;
     const unsigned long long *d_ids = nullptr;
     if (problem_ids) {  // every window keeps its own key, whatever its position in this batch

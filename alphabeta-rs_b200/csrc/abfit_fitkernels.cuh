@@ -743,6 +743,8 @@ __device__ __forceinline__ void fit_starts_body_v2(const DevicePools &P, const W
             if (((idle >> lane) & 1u) && rank < take) {
                 const int id = q.next + rank;
                 const double *sx = simplices + ((size_t)q.prob * n_starts + id) * 20;
+                // read-only path although, under the upload watch, a copy engine is still writing other windows'
+                // simplices: see DESIGN §2.10 for why no stale sector can be read
 #pragma unroll
                 for (int k = 0; k < 20; ++k) S.X[k * 32] = sx[k];
                 nm_begin(L, S, id);
