@@ -94,6 +94,9 @@ def _load() -> C.CDLL:
         "abfit_site_boot_batch_device": (C.c_int, [vp, PP, i32, vp, vp, vp, vp, i32, i64, vp, dbl, i64, vp, i32, u64, u64, vp,
                                                    i32, dbl, u32, vp, vp, vp, vp, vp]),
         "abfit_gen_vary_vertices_batch": (None, [u64, u64, i32, i32, vp, vp]),
+        "abfit_gen_param_boot_seeds": (None, [u64, u64, i32, vp]),
+        "abfit_param_boot_batch": (C.c_int, [vp, vp, PP, i32, vp, vp, dbl, vp, i32, u64, u64, vp, i32, dbl, u32, vp, vp, vp,
+                                             vp, vp, vp, vp, vp]),
         "abfit_device_count": (C.c_int, []),
         "abfit_alphabeta_batch_multi": (C.c_int, [vp, i32, vp, i32, i32, vp, i32, vp, u64, u64, vp, i32, i32, dbl, u32, vp, vp, vp, vp, vp, vp]),
         "abfit_divergence_multi": (C.c_int, [vp, i32, vp, vp, vp, i32, i64, vp, i32, dbl, vp, vp, vp, vp, vp, vp]),
@@ -180,6 +183,7 @@ EXPORTED_SYMBOLS = (
     "abfit_sim_tree_build abfit_sim_tree_from_arrays abfit_sim_tree_info abfit_sim_tree_pairs abfit_sim_tree_thresholds "
     "abfit_sim_tree_free abfit_sim_equilibrium abfit_simulate abfit_simulate_device "
     "abfit_gen_site_boot_counts abfit_site_boot_batch abfit_site_boot_batch_device "
+    "abfit_gen_param_boot_seeds abfit_param_boot_batch "
     "abfit_parse_region_line abfit_region_ranges abfit_region_divergence abfit_region_divergence_device"
 ).split()
 
@@ -226,6 +230,13 @@ def gen_resample_idx(seed: int, problem_id: int, n_boot: int, n_pairs: int) -> n
     """residual resampling with replacement (src/boot_model.rs:43-48) -> int32 [n_boot,n_pairs]."""
     out = np.empty((n_boot, n_pairs), dtype=np.int32)
     _lib.abfit_gen_resample_idx(seed, problem_id, n_boot, n_pairs, _ptr(out))
+    return out
+
+
+def gen_param_boot_seeds(seed: int, problem_key: int, n_boot: int) -> np.ndarray:
+    """the simulator seeds of a window's parametric-bootstrap replicates (generator stream 6) -> u64 [n_boot]"""
+    out = np.empty(n_boot, dtype=np.uint64)
+    _lib.abfit_gen_param_boot_seeds(seed, problem_key, n_boot, _ptr(out))
     return out
 
 
@@ -598,6 +609,46 @@ class Context:
         return self._site_boot(_lib.abfit_site_boot_batch_device, probs, pairs,
                                (C.c_void_p(d_status), C.c_void_p(d_post), C.c_void_p(d_meth)), S, L, seg_offsets, best,
                                n_boot, seed, block_sites, thr, first_problem_id, problem_ids, max_iters, sd_tol, flags)
+
+    # -- parametric bootstrap and goodness of fit (include/abfit.h, abfit_param_boot_batch) --------
+    def parametric_bootstrap(self, tree: "SimTree", probs: Sequence[Problem], n_sites, missing, best, n_boot, seed,
+                             thr=0.99, first_problem_id=0, problem_ids=None, max_iters=1000, sd_tol=DBL_EPSILON, flags=0):
+        """Parametric bootstrap of fitted windows that share the forest `tree` (abfit_param_boot_batch): replicate b of
+        window p is simulated from best[p]'s model (alpha, beta, weight, intercept) with probs[p].p0uu, n_sites[p] sites
+        and the per-sample missing rates missing[p] ([n_probs, n_samples], or None), refitted from [best, vary x 4], and
+        the observed LSE best[p]["lse"] is ranked among the replicates'.  -> dict(rows [n_probs, n_boot, 7], fits,
+        analysis [n_probs, 32], dstar [n_probs, n_boot, n_pairs], lse_star [n_probs, n_boot], gof_p [n_probs],
+        window_status [n_probs] (1: the fitted model cannot be simulated), nan_reps [n_probs])"""
+        n_probs = len(probs)
+        R, S = tree.n_pairs, tree.n_samples
+        n_sites = np.ascontiguousarray(n_sites, dtype=np.int64).reshape(-1)
+        best = np.ascontiguousarray(best, dtype=FIT_DTYPE).reshape(-1)
+        ids = None if problem_ids is None else np.ascontiguousarray(problem_ids, dtype=np.uint64).reshape(-1)
+        if n_sites.shape != (n_probs,):
+            raise ValueError(f"n_sites needs {n_probs} entries, got {n_sites.size}")
+        if best.shape != (n_probs,):
+            raise ValueError(f"best needs {n_probs} entries, got {best.size}")
+        if ids is not None and ids.shape != (n_probs,):
+            raise ValueError(f"problem_ids needs {n_probs} entries, got {ids.size}")
+        if missing is not None:
+            missing = np.ascontiguousarray(missing, dtype=np.float64)
+            if missing.shape != (n_probs, S):
+                raise ValueError(f"missing must be [{n_probs}, {S}], got {list(missing.shape)}")
+        n_boot = int(n_boot)
+        rows = np.empty((n_probs, n_boot, 7))
+        fits = np.zeros((n_probs, n_boot), dtype=FIT_DTYPE)
+        analysis = np.empty((n_probs, 32))
+        dstar = np.empty((n_probs, n_boot, R))
+        lse_star = np.empty((n_probs, n_boot))
+        gof_p = np.empty(n_probs)
+        wstat = np.zeros(n_probs, dtype=np.int32)
+        nan_reps = np.zeros(n_probs, dtype=np.int32)
+        _check(_lib.abfit_param_boot_batch(self._h, tree._h, _pack_problems(probs), n_probs, _ptr(n_sites), _ptr(missing),
+                                           thr, _ptr(best), n_boot, seed, first_problem_id, _ptr(ids), max_iters, sd_tol,
+                                           flags, _ptr(rows), _ptr(fits), _ptr(analysis), _ptr(dstar), _ptr(lse_star),
+                                           _ptr(gof_p), _ptr(wstat), _ptr(nan_reps)))
+        return {"rows": rows, "fits": fits, "analysis": analysis, "dstar": dstar, "lse_star": lse_star, "gof_p": gof_p,
+                "window_status": wstat, "nan_reps": nan_reps}
 
     # -- genomic regions (include/abfit.h, abfit_region_divergence) -------------------------------
     def _region_div(self, fn, inputs, S, L, lo, hi, thr, extra=()):

@@ -15,6 +15,7 @@
 
 #include "abfit_jit.h"
 #include "abfit_plan.h"
+#include "abfit_psim.cuh"
 
 namespace abfit {
 
@@ -1645,6 +1646,79 @@ void abfit_gen_site_boot_counts(uint64_t seed, uint64_t problem_key, int32_t n_b
             ++counts_out[(size_t)b * n_blocks + site_boot_block(seed, problem_key, (uint64_t)b, (uint64_t)d, n_blocks)];
 }
 
+// The refit of given D* replicates, shared by the site-block and the parametric bootstrap: d_dstar [pair_off * n_boot +
+// b * n_pairs + i] and d_nan [n_probs][n_boot] (1: a pair of the replicate has no valid site) are on the device, filled
+// on the context stream.  Replicates start from [best, vary x 4], vary drawn on the device from the window keys (d_ids,
+// else first_problem_id + p), and run on the mapping abfit_boot_batch's planner picks for b's pedigrees.
+static int refit_given_dstar(abfit_ctx *ctx, abfit_batch *b, int32_t n_probs, const abfit_fit *best, int32_t n_boot,
+                             uint64_t seed, uint64_t first_problem_id, const unsigned long long *d_ids, const double *d_dstar,
+                             const uint8_t *d_nan, int64_t total_pairs, int32_t max_iters, double sd_tol, uint32_t flags,
+                             double *rows_out, abfit_fit *fits_out, double *analysis_out, double *dstar_out,
+                             int32_t *nan_reps_out)
+{
+    cudaStream_t st = ctx->stream;
+    // the mapping abfit_boot_batch's planner picks for these pedigrees: warp-per-fit, else the stored-D* tile
+    const int n_sm = ctx->prop.multiProcessorCount;
+    std::vector<WorkItem> items = b->shape.wide ? make_items_wide(b->hp, n_boot, n_sm, false)
+                                                : make_items(b->hp, n_boot, n_sm, 1, false);
+    DevBuf<WorkItem> d_items;
+    DevBuf<double> d_rows, d_tile, d_an, d_an_scratch;
+    DevBuf<abfit_fit> d_fits;
+    if (int rc = d_items.ensure(items.size())) return rc;
+    if (int rc = d_rows.ensure((size_t)n_probs * n_boot * 7)) return rc;
+    if (int rc = d_fits.ensure((size_t)n_probs * n_boot)) return rc;
+    if (int rc = b->d_best.ensure(n_probs)) return rc;
+    if (int rc = b->d_vary.ensure((size_t)n_probs * n_boot * 16)) return rc;
+    if (!b->shape.wide)
+        if (int rc = d_tile.ensure((items.size() + 1) * (size_t)b->hp.max_pairs * 32)) return rc;
+    const bool dev_stats = analysis_out && n_boot >= 2;
+    if (dev_stats) {
+        if (int rc = d_an.ensure((size_t)n_probs * 32)) return rc;
+        if (int rc = d_an_scratch.ensure((size_t)n_probs * 8 * n_boot)) return rc;
+    }
+    BigScratch big;
+    if (!b->shape.wide)
+        if (int rc = big_scratch(b, std::max<size_t>(items.size(), 1), big)) return rc;
+    if (!items.empty())
+        ABFIT_CUDA(cudaMemcpyAsync(d_items.p, items.data(), items.size() * sizeof(WorkItem), cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemcpyAsync(b->d_best.p, best, (size_t)n_probs * sizeof(abfit_fit), cudaMemcpyHostToDevice, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_rows.p, 0xFF, (size_t)n_probs * n_boot * 7 * 8, st));
+    ABFIT_CUDA(cudaMemsetAsync(d_fits.p, 0xFF, (size_t)n_probs * n_boot * sizeof(abfit_fit), st));
+    ABFIT_CUDA(cudaMemsetAsync(b->d_evals_boot.p, 0, (size_t)n_probs * 8, st));
+    if (int rc = launch_gen_vary(st, seed, first_problem_id, d_ids, n_probs, n_boot, b->d_best.p, b->d_vary.p)) return rc;
+    const NMParams nm = nm_params(max_iters, sd_tol, flags);
+    if (b->shape.wide) {
+        if (int rc = launch_fit_boot_wide_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar,
+                                                b->d_vary.p, nm, d_rows.p, d_fits.p, b->d_evals_boot.p, b->shape.smem_wide))
+            return rc;
+    } else if (int rc = launch_fit_boot_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar,
+                                              b->d_vary.p, d_tile.p, (int64_t)b->hp.max_pairs * 32, nm, d_rows.p, d_fits.p,
+                                              b->d_evals_boot.p, b->shape.smem_boot, big)) {
+        return rc;
+    }
+    if (dev_stats) {
+        if (int rc = launch_analyze(st, d_rows.p, n_probs, n_boot, d_an.p, d_an_scratch.p)) return rc;
+        ABFIT_CUDA(cudaMemcpyAsync(analysis_out, d_an.p, (size_t)n_probs * 32 * 8, cudaMemcpyDeviceToHost, st));
+    }
+    std::vector<uint8_t> nan_rep((size_t)n_probs * n_boot);
+    ABFIT_CUDA(cudaMemcpyAsync(rows_out, d_rows.p, (size_t)n_probs * n_boot * 7 * 8, cudaMemcpyDeviceToHost, st));
+    if (fits_out)
+        ABFIT_CUDA(cudaMemcpyAsync(fits_out, d_fits.p, (size_t)n_probs * n_boot * sizeof(abfit_fit), cudaMemcpyDeviceToHost, st));
+    if (dstar_out)
+        ABFIT_CUDA(cudaMemcpyAsync(dstar_out, d_dstar, (size_t)total_pairs * n_boot * 8, cudaMemcpyDeviceToHost, st));
+    ABFIT_CUDA(cudaMemcpyAsync(nan_rep.data(), d_nan, nan_rep.size(), cudaMemcpyDeviceToHost, st));
+    ABFIT_CUDA(cudaStreamSynchronize(st));
+    if (nan_reps_out)
+        for (int p = 0; p < n_probs; ++p) {
+            int32_t n = 0;
+            for (int k = 0; k < n_boot; ++k) n += nan_rep[(size_t)p * n_boot + k];
+            nan_reps_out[p] = n;
+        }
+    if (analysis_out && !dev_stats)
+        for (int p = 0; p < n_probs; ++p) abfit_analyze(rows_out + (size_t)p * n_boot * 7, n_boot, analysis_out + (size_t)p * 32);
+    return 0;
+}
+
 static int site_boot_impl(abfit_ctx *ctx, bool device_inputs, const abfit_problem *probs, int32_t n_probs,
                           const int32_t *pairs, const uint8_t *status, const double *posterior_max, const double *meth_lvl,
                           int32_t S, int64_t L, const int64_t *seg, double thr, int64_t block_sites, const abfit_fit *best,
@@ -1772,10 +1846,6 @@ static int site_boot_impl(abfit_ctx *ctx, bool device_inputs, const abfit_proble
         ABFIT_CUDA(cudaStreamSynchronize(st));  // the temporaries are freed at the end of this scope
     }
 
-    // the mapping abfit_boot_batch's planner picks for these pedigrees: warp-per-fit, else the stored-D* tile
-    const int n_sm = ctx->prop.multiProcessorCount;
-    std::vector<WorkItem> items = b->shape.wide ? make_items_wide(b->hp, n_boot, n_sm, false)
-                                                : make_items(b->hp, n_boot, n_sm, 1, false);
     std::vector<SiteBootItem> ditems;
     {
         int64_t off = 0;
@@ -1795,88 +1865,35 @@ static int site_boot_impl(abfit_ctx *ctx, bool device_inputs, const abfit_proble
             off += np;
         }
     }
-    DevBuf<WorkItem> d_items;
     DevBuf<SiteBootItem> d_ditems;
     DevBuf<long long> d_blk_off;
     DevBuf<int32_t> d_row_pair;
     DevBuf<uint32_t> d_counts;
-    DevBuf<double> d_dstar, d_rows, d_tile, d_an, d_an_scratch;
+    DevBuf<double> d_dstar;
     DevBuf<uint8_t> d_nan;
-    DevBuf<abfit_fit> d_fits;
-    if (int rc = d_items.ensure(items.size())) return rc;
     if (int rc = d_ditems.ensure(ditems.size())) return rc;
     if (int rc = d_blk_off.ensure(blk_off.size())) return rc;
     if (int rc = d_row_pair.ensure(row_pair.size())) return rc;
     if (int rc = d_counts.ensure((size_t)n_blk * n_boot)) return rc;
     if (int rc = d_dstar.ensure((size_t)total_pairs * n_boot)) return rc;
     if (int rc = d_nan.ensure((size_t)n_probs * n_boot)) return rc;
-    if (int rc = d_rows.ensure((size_t)n_probs * n_boot * 7)) return rc;
-    if (int rc = d_fits.ensure((size_t)n_probs * n_boot)) return rc;
-    if (int rc = b->d_best.ensure(n_probs)) return rc;
-    if (int rc = b->d_vary.ensure((size_t)n_probs * n_boot * 16)) return rc;
-    if (!b->shape.wide)
-        if (int rc = d_tile.ensure((items.size() + 1) * (size_t)b->hp.max_pairs * 32)) return rc;
-    const bool dev_stats = analysis_out && n_boot >= 2;
-    if (dev_stats) {
-        if (int rc = d_an.ensure((size_t)n_probs * 32)) return rc;
-        if (int rc = d_an_scratch.ensure((size_t)n_probs * 8 * n_boot)) return rc;
-    }
-    BigScratch big;
-    if (!b->shape.wide)
-        if (int rc = big_scratch(b, std::max<size_t>(items.size(), 1), big)) return rc;
     const unsigned long long *d_ids = nullptr;
     if (problem_ids) {
         if (int rc = b->d_ids.ensure(n_probs)) return rc;
         ABFIT_CUDA(cudaMemcpyAsync(b->d_ids.p, problem_ids, (size_t)n_probs * 8, cudaMemcpyHostToDevice, st));
         d_ids = b->d_ids.p;
     }
-    if (!items.empty())
-        ABFIT_CUDA(cudaMemcpyAsync(d_items.p, items.data(), items.size() * sizeof(WorkItem), cudaMemcpyHostToDevice, st));
     ABFIT_CUDA(cudaMemcpyAsync(d_ditems.p, ditems.data(), ditems.size() * sizeof(SiteBootItem), cudaMemcpyHostToDevice, st));
     ABFIT_CUDA(cudaMemcpyAsync(d_blk_off.p, blk_off.data(), blk_off.size() * 8, cudaMemcpyHostToDevice, st));
     ABFIT_CUDA(cudaMemcpyAsync(d_row_pair.p, row_pair.data(), row_pair.size() * 4, cudaMemcpyHostToDevice, st));
-    ABFIT_CUDA(cudaMemcpyAsync(b->d_best.p, best, (size_t)n_probs * sizeof(abfit_fit), cudaMemcpyHostToDevice, st));
     ABFIT_CUDA(cudaMemsetAsync(d_counts.p, 0, (size_t)n_blk * n_boot * 4, st));
     ABFIT_CUDA(cudaMemsetAsync(d_nan.p, 0, (size_t)n_probs * n_boot, st));
-    ABFIT_CUDA(cudaMemsetAsync(d_rows.p, 0xFF, (size_t)n_probs * n_boot * 7 * 8, st));
-    ABFIT_CUDA(cudaMemsetAsync(d_fits.p, 0xFF, (size_t)n_probs * n_boot * sizeof(abfit_fit), st));
-    ABFIT_CUDA(cudaMemsetAsync(b->d_evals_boot.p, 0, (size_t)n_probs * 8, st));
-    if (int rc = launch_gen_vary(st, seed, first_problem_id, d_ids, n_probs, n_boot, b->d_best.p, b->d_vary.p)) return rc;
     if (int rc = launch_siteboot_counts(st, seed, first_problem_id, d_ids, d_blk_off.p, n_probs, n_boot, n_blk, d_counts.p)) return rc;
     if (int rc = launch_siteboot_dstar(st, d_ditems.p, (int)ditems.size(), n_boot, d_part.p, P, d_counts.p, d_row_pair.p,
                                        d_dstar.p, d_nan.p))
         return rc;
-    const NMParams nm = nm_params(max_iters, sd_tol, flags);
-    if (b->shape.wide) {
-        if (int rc = launch_fit_boot_wide_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar.p,
-                                                b->d_vary.p, nm, d_rows.p, d_fits.p, b->d_evals_boot.p, b->shape.smem_wide))
-            return rc;
-    } else if (int rc = launch_fit_boot_given(st, b->pools, d_items.p, (int)items.size(), n_boot, b->d_best.p, d_dstar.p,
-                                              b->d_vary.p, d_tile.p, (int64_t)b->hp.max_pairs * 32, nm, d_rows.p, d_fits.p,
-                                              b->d_evals_boot.p, b->shape.smem_boot, big)) {
-        return rc;
-    }
-    if (dev_stats) {
-        if (int rc = launch_analyze(st, d_rows.p, n_probs, n_boot, d_an.p, d_an_scratch.p)) return rc;
-        ABFIT_CUDA(cudaMemcpyAsync(analysis_out, d_an.p, (size_t)n_probs * 32 * 8, cudaMemcpyDeviceToHost, st));
-    }
-    std::vector<uint8_t> nan_rep((size_t)n_probs * n_boot);
-    ABFIT_CUDA(cudaMemcpyAsync(rows_out, d_rows.p, (size_t)n_probs * n_boot * 7 * 8, cudaMemcpyDeviceToHost, st));
-    if (fits_out)
-        ABFIT_CUDA(cudaMemcpyAsync(fits_out, d_fits.p, (size_t)n_probs * n_boot * sizeof(abfit_fit), cudaMemcpyDeviceToHost, st));
-    if (dstar_out)
-        ABFIT_CUDA(cudaMemcpyAsync(dstar_out, d_dstar.p, (size_t)total_pairs * n_boot * 8, cudaMemcpyDeviceToHost, st));
-    ABFIT_CUDA(cudaMemcpyAsync(nan_rep.data(), d_nan.p, nan_rep.size(), cudaMemcpyDeviceToHost, st));
-    ABFIT_CUDA(cudaStreamSynchronize(st));
-    if (nan_reps_out)
-        for (int p = 0; p < n_probs; ++p) {
-            int32_t n = 0;
-            for (int k = 0; k < n_boot; ++k) n += nan_rep[(size_t)p * n_boot + k];
-            nan_reps_out[p] = n;
-        }
-    if (analysis_out && !dev_stats)
-        for (int p = 0; p < n_probs; ++p) abfit_analyze(rows_out + (size_t)p * n_boot * 7, n_boot, analysis_out + (size_t)p * 32);
-    return 0;
+    return refit_given_dstar(ctx, b, n_probs, best, n_boot, seed, first_problem_id, d_ids, d_dstar.p, d_nan.p, total_pairs,
+                             max_iters, sd_tol, flags, rows_out, fits_out, analysis_out, dstar_out, nan_reps_out);
 }
 
 int abfit_site_boot_batch(abfit_ctx *ctx, const abfit_problem *probs, int32_t n_probs, const int32_t *pairs,
@@ -1902,6 +1919,211 @@ int abfit_site_boot_batch_device(abfit_ctx *ctx, const abfit_problem *probs, int
     return site_boot_impl(ctx, true, probs, n_probs, pairs, d_status, d_posterior_max, d_meth_lvl, S, L, seg_offsets, thr,
                           block_sites, best, n_boot, seed, first_problem_id, problem_ids, max_iters, sd_tol, flags, rows_out,
                           fits_out, analysis_out, dstar_out, nan_reps_out);
+}
+
+// ---------------------------------------------------------------------------------------
+// parametric bootstrap: replicates simulated from every window's fitted model and counted to exact per-row sums in one
+// kernel (k_psim_counts) -> D* = D_sim + theta3 (k_psim_dstar) -> the site bootstrap's refit of the given D*
+// ---------------------------------------------------------------------------------------
+void abfit_gen_param_boot_seeds(uint64_t seed, uint64_t problem_key, int32_t n_boot, uint64_t *seeds_out)
+{
+    if (!seeds_out) return;
+    for (int32_t b = 0; b < n_boot; ++b) seeds_out[b] = param_boot_seed(seed, problem_key, (uint64_t)b);
+}
+
+int abfit_param_boot_batch(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_problem *probs, int32_t n_probs,
+                           const int64_t *n_sites, const double *missing, double thr, const abfit_fit *best, int32_t n_boot,
+                           uint64_t seed, uint64_t first_problem_id, const uint64_t *problem_ids, int32_t max_iters,
+                           double sd_tol, uint32_t flags, double *rows_out, abfit_fit *fits_out, double *analysis_out,
+                           double *dstar_out, double *lse_star_out, double *gof_p_out, int32_t *window_status_out,
+                           int32_t *nan_reps_out)
+{
+    auto refuse = [](int rc, const std::string &m) {
+        set_error("parametric bootstrap: " + m);
+        return rc;
+    };
+    // every refusal that needs no device comes first
+    if (!tree || !probs || n_probs <= 0 || !n_sites || !best || !rows_out || n_boot <= 0 || max_iters < 0)
+        return refuse(ABFIT_ERR_ARG, "missing or out-of-range argument");
+    if (n_boot > 65535) return refuse(ABFIT_ERR_TOO_LARGE, "at most 65535 replicates per call");
+    int32_t n_nodes = 0, S = 0, R = 0;
+    abfit_sim_tree_info(tree, &n_nodes, &S, &R);
+    if (R <= 0) return refuse(ABFIT_ERR_ARG, "the forest has no pair of sampled nodes in one tree");
+    if (S > PSIM_MAX_S)
+        return refuse(ABFIT_ERR_TOO_LARGE, std::to_string(S) + " sampled nodes, at most " + std::to_string(PSIM_MAX_S));
+    std::vector<double> tp((size_t)R * 5);
+    abfit_sim_tree_pairs(tree, tp.data(), R);
+    for (int p = 0; p < n_probs; ++p) {
+        if (probs[p].n_pairs != R || !probs[p].pedigree)
+            return refuse(ABFIT_ERR_ARG, "problem " + std::to_string(p) + " has " + std::to_string(probs[p].n_pairs) +
+                                             " pedigree rows, the forest " + std::to_string(R));
+        for (int r = 0; r < R; ++r)
+            for (int c = 0; c < 3; ++c)
+                if (!(probs[p].pedigree[(size_t)r * 4 + c] == tp[(size_t)r * 5 + 2 + c]))
+                    return refuse(ABFIT_ERR_ARG, "problem " + std::to_string(p) + ", pedigree row " + std::to_string(r) +
+                                                     ": (t0, t1, t2) differ from the forest's pair rows");
+        if (n_sites[p] <= 0) return refuse(ABFIT_ERR_ARG, "window " + std::to_string(p) + " has no sites");
+        if (n_sites[p] >= ((int64_t)1 << 31))
+            return refuse(ABFIT_ERR_TOO_LARGE, "window " + std::to_string(p) + " has 2^31 sites or more");
+        if (missing)
+            for (int s = 0; s < S; ++s) {
+                const double m = missing[(size_t)p * S + s];
+                if (!(m >= 0.0 && m <= 1.0))
+                    return refuse(ABFIT_ERR_ARG, "window " + std::to_string(p) + ", sample " + std::to_string(s) +
+                                                     ": missing rate outside [0, 1]");
+            }
+    }
+    if (!ctx) return refuse(ABFIT_ERR_ARG, "no context");
+    const uint64_t smem = psim_smem_bytes(n_nodes, S, R);
+    if (smem > (uint64_t)ctx->smem_optin)
+        return refuse(ABFIT_ERR_TOO_LARGE, std::to_string(n_nodes) + " nodes, " + std::to_string(S) + " samples and " +
+                                               std::to_string(R) + " rows need " + std::to_string(smem) +
+                                               " B of shared memory per block, " + std::to_string(ctx->smem_optin) +
+                                               " B are available");
+    // windows whose fitted model cannot be simulated get status 1 and no launch
+    auto in01 = [](double x) { return x >= 0.0 && x <= 1.0; };
+    std::vector<int32_t> valid;
+    std::vector<int32_t> wstat(n_probs, 0);
+    for (int p = 0; p < n_probs; ++p) {
+        const double *th = best[p].theta;
+        const bool ok = in01(th[0]) && in01(th[1]) && in01(th[2]) && in01(probs[p].p0uu) && std::isfinite(th[3]);
+        wstat[p] = ok ? 0 : 1;
+        if (ok) valid.push_back(p);
+    }
+    const int nv = (int)valid.size();
+    // host tables: walk, per-window thresholds and missing rates, tile items
+    std::vector<int32_t> parent_pos, node_id, row_pos, row_ij(R);
+    sim_walk(tree, parent_pos, node_id, row_pos);
+    for (int r = 0; r < R; ++r) row_ij[r] = (int32_t)tp[(size_t)r * 5] | ((int32_t)tp[(size_t)r * 5 + 1] << 16);
+    std::vector<double> thr6((size_t)nv * n_nodes * 6), miss((size_t)nv * S, 0.0), theta3(nv);
+    std::vector<unsigned long long> keys(nv);
+    std::vector<abfit_problem> vprobs(nv);
+    std::vector<abfit_fit> vbest(nv);
+    std::vector<PsimItem> items;
+    for (int q = 0; q < nv; ++q) {
+        const int p = valid[q];
+        const abfit_sim_params prm{best[p].theta[0], best[p].theta[1], best[p].theta[2], probs[p].p0uu, 0.0, 0};
+        if (int rc = sim_thresholds_walk(tree, &prm, thr6.data() + (size_t)q * n_nodes * 6)) return rc;
+        if (missing) std::copy(missing + (size_t)p * S, missing + (size_t)(p + 1) * S, miss.begin() + (size_t)q * S);
+        theta3[q] = best[p].theta[3];
+        keys[q] = problem_ids ? problem_ids[p] : first_problem_id + (uint64_t)p;
+        vprobs[q] = probs[p];
+        vbest[q] = best[p];
+        const int64_t tiles = (n_sites[p] + PSIM_TILE - 1) / PSIM_TILE;
+        for (int64_t t0 = 0; t0 < tiles; t0 += PSIM_MAX_TILES)
+            items.push_back(PsimItem{q, (int32_t)std::min<int64_t>(PSIM_MAX_TILES, tiles - t0), t0, n_sites[p]});
+    }
+    if (items.size() > (size_t)INT32_MAX) return refuse(ABFIT_ERR_TOO_LARGE, "2^31 tiles or more in one call");
+    const int64_t total_rows = (int64_t)nv * R;
+    // results of the windows that run: straight into the caller's arrays when every window runs, else compacted
+    const bool all = nv == n_probs;
+    std::vector<double> c_rows, c_an, c_dstar;
+    std::vector<abfit_fit> c_fits;
+    std::vector<int32_t> c_nan(nv);
+    if (!all) {
+        c_rows.resize((size_t)nv * n_boot * 7);
+        if (analysis_out) c_an.resize((size_t)nv * 32);
+        if (dstar_out) c_dstar.resize((size_t)total_rows * n_boot);
+    }
+    if (!fits_out || !all) c_fits.resize((size_t)nv * n_boot);
+    abfit_fit *fits = all && fits_out ? fits_out : c_fits.data();
+    if (nv > 0) {
+        ABFIT_CUDA(cudaSetDevice(ctx->device));
+        cudaStream_t st = ctx->stream;
+        abfit_batch *b = nullptr;
+        if (int rc = workspace(ctx, vprobs.data(), nv, &b)) return rc;
+        const size_t need = (size_t)total_rows * n_boot * 8 + (size_t)nv * n_boot * (7 * 8 + sizeof(abfit_fit) + 16 * 8 + 8 * 8 + 1) +
+                            thr6.size() * 8 + miss.size() * 8 + items.size() * sizeof(PsimItem) +
+                            (size_t)b->hp.max_pairs * 32 * 8 * (size_t)(4 * ctx->prop.multiProcessorCount + 1) + ((size_t)64 << 20);
+        size_t fr = 0, tot = 0;
+        ABFIT_CUDA(cudaMemGetInfo(&fr, &tot));
+        if (need > fr)
+            return refuse(ABFIT_ERR_TOO_LARGE, std::to_string(nv) + " windows x " + std::to_string(n_boot) + " replicates x " +
+                                                   std::to_string(R) + " rows need about " + std::to_string(need >> 20) +
+                                                   " MiB of device memory, " + std::to_string(fr >> 20) + " MiB are free");
+        DevBuf<PsimItem> d_items;
+        DevBuf<double> d_thr6, d_miss, d_theta3;
+        DevBuf<int32_t> d_parent, d_node, d_rowpos, d_rowij;
+        DevBuf<unsigned long long> d_keys, d_sums;
+        DevBuf<uint8_t> d_nan;
+        if (int rc = d_items.ensure(items.size())) return rc;
+        if (int rc = d_thr6.ensure(thr6.size())) return rc;
+        if (int rc = d_miss.ensure(miss.size())) return rc;
+        if (int rc = d_theta3.ensure(nv)) return rc;
+        if (int rc = d_parent.ensure(n_nodes)) return rc;
+        if (int rc = d_node.ensure(n_nodes)) return rc;
+        if (int rc = d_rowpos.ensure(S)) return rc;
+        if (int rc = d_rowij.ensure(R)) return rc;
+        if (int rc = d_keys.ensure(nv)) return rc;
+        if (int rc = d_sums.ensure((size_t)total_rows * n_boot)) return rc;
+        if (int rc = d_nan.ensure((size_t)nv * n_boot)) return rc;
+        ABFIT_CUDA(cudaMemcpyAsync(d_items.p, items.data(), items.size() * sizeof(PsimItem), cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_thr6.p, thr6.data(), thr6.size() * 8, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_miss.p, miss.data(), miss.size() * 8, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_theta3.p, theta3.data(), (size_t)nv * 8, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_parent.p, parent_pos.data(), (size_t)n_nodes * 4, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_node.p, node_id.data(), (size_t)n_nodes * 4, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_rowpos.p, row_pos.data(), (size_t)S * 4, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_rowij.p, row_ij.data(), (size_t)R * 4, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemcpyAsync(d_keys.p, keys.data(), (size_t)nv * 8, cudaMemcpyHostToDevice, st));
+        ABFIT_CUDA(cudaMemsetAsync(d_sums.p, 0, (size_t)total_rows * n_boot * 8, st));
+        ABFIT_CUDA(cudaMemsetAsync(d_nan.p, 0, (size_t)nv * n_boot, st));
+        if (int rc = launch_psim_counts(st, d_items.p, (int)items.size(), d_thr6.p, d_parent.p, d_node.p, n_nodes, d_rowpos.p,
+                                        d_miss.p, S, d_rowij.p, R, thr, seed, d_keys.p, n_boot, d_sums.p))
+            return rc;
+        if (int rc = launch_psim_dstar(st, d_sums.p, total_rows * n_boot, R, n_boot, d_theta3.p, d_nan.p)) return rc;
+        if (int rc = refit_given_dstar(ctx, b, nv, vbest.data(), n_boot, seed, 0, d_keys.p,
+                                       reinterpret_cast<const double *>(d_sums.p), d_nan.p, total_rows, max_iters, sd_tol, flags,
+                                       all ? rows_out : c_rows.data(), fits, all ? analysis_out : (analysis_out ? c_an.data() : nullptr),
+                                       all ? dstar_out : (dstar_out ? c_dstar.data() : nullptr), c_nan.data()))
+            return rc;
+    }
+    // scatter the windows that ran; the others get NaN
+    const double qnan = std::nan("");
+    for (int p = 0, q = 0; p < n_probs; ++p) {
+        const bool ran = wstat[p] == 0;
+        if (!all) {
+            double *ro = rows_out + (size_t)p * n_boot * 7;
+            if (ran) std::copy(c_rows.begin() + (size_t)q * n_boot * 7, c_rows.begin() + (size_t)(q + 1) * n_boot * 7, ro);
+            else std::fill(ro, ro + (size_t)n_boot * 7, qnan);
+            if (analysis_out) {
+                double *ao = analysis_out + (size_t)p * 32;
+                if (ran) std::copy(c_an.begin() + (size_t)q * 32, c_an.begin() + (size_t)(q + 1) * 32, ao);
+                else std::fill(ao, ao + 32, qnan);
+            }
+            if (dstar_out) {
+                double *d = dstar_out + (size_t)p * R * n_boot;
+                if (ran) std::copy(c_dstar.begin() + (size_t)q * R * n_boot, c_dstar.begin() + (size_t)(q + 1) * R * n_boot, d);
+                else std::fill(d, d + (size_t)R * n_boot, qnan);
+            }
+            if (fits_out)
+                for (int k = 0; k < n_boot; ++k) {
+                    abfit_fit &f = fits_out[(size_t)p * n_boot + k];
+                    if (ran) {
+                        f = c_fits[(size_t)q * n_boot + k];
+                        continue;
+                    }
+                    f.theta[0] = f.theta[1] = f.theta[2] = f.theta[3] = f.cost = f.lse = qnan;
+                    f.iters = f.evals = 0;
+                    f.status = ABFIT_FIT_NAN;
+                    f.start_id = k;
+                }
+        }
+        int32_t fitted = 0, ge = 0;
+        for (int k = 0; k < n_boot; ++k) {
+            const double l = ran ? fits[(size_t)q * n_boot + k].lse : qnan;
+            if (lse_star_out) lse_star_out[(size_t)p * n_boot + k] = l;
+            if (ran && fits[(size_t)q * n_boot + k].status != ABFIT_FIT_NAN) {
+                ++fitted;
+                ge += l >= best[p].lse ? 1 : 0;
+            }
+        }
+        if (gof_p_out) gof_p_out[p] = ran ? (1.0 + (double)ge) / (1.0 + (double)fitted) : qnan;
+        if (nan_reps_out) nan_reps_out[p] = ran ? c_nan[q] : 0;
+        if (window_status_out) window_status_out[p] = wstat[p];
+        if (ran) ++q;
+    }
+    return 0;
 }
 
 int abfit_simulate(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site, int64_t L,

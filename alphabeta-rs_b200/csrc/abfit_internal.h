@@ -180,5 +180,26 @@ int read_node_edge_lists(const char *nodelist_path, const char *edgelist_path, s
 // device arrays (device_out) or host arrays (staged through device buffers); kernel_ms optional
 int run_simulate(cudaStream_t st, int n_sms, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
                  int64_t L, uint8_t *status, double *posterior_max, double *meth_lvl, bool device_out, float *kernel_ms);
+// the walk order of k_simulate: per walk position its parent's position (-1: root) and node index; per sampled row its
+// walk position
+void sim_walk(const abfit_sim_tree *tree, std::vector<int32_t> &parent_pos, std::vector<int32_t> &node_id,
+              std::vector<int32_t> &row_pos);
+// abfit_sim_tree_thresholds in walk order: out [n_nodes][6] (ABFIT_ERR_ARG for parameters outside [0, 1])
+int sim_thresholds_walk(const abfit_sim_tree *tree, const abfit_sim_params *params, double *out);
+
+// ---- parametric bootstrap (abfit_psim.cu) -------------------------------------------------
+struct PsimItem {
+    int32_t prob, n_tiles;  // tiles [tile0, tile0 + n_tiles) of window prob, n_tiles <= PSIM_MAX_TILES
+    int64_t tile0;
+    int64_t L;              // sites of the window
+};
+// sums [n_probs][n_boot][R] packed cnt << 32 | diff, zeroed first; grid = n_items x n_boot
+int launch_psim_counts(cudaStream_t st, const PsimItem *items, int n_items, const double *thr6, const int32_t *parent_pos,
+                       const int32_t *node_id, int n, const int32_t *row_pos, const double *miss, int S,
+                       const int32_t *row_ij, int R, double thr, uint64_t seed, const unsigned long long *keys, int n_boot,
+                       unsigned long long *sums);
+// in place: sums -> D* = diff / (2.0 * cnt) + theta3[p] (doubles, layout of the site bootstrap's D*); nan_rep zeroed first
+int launch_psim_dstar(cudaStream_t st, unsigned long long *sums, int64_t total, int R, int n_boot, const double *theta3,
+                      uint8_t *nan_rep);
 
 }  // namespace abfit

@@ -55,4 +55,12 @@ ABFIT_HD inline int32_t site_boot_block(uint64_t seed, uint64_t problem_id, uint
     return k;
 }
 
+// parametric bootstrap: the simulator seed of replicate b of window problem_id (stream 6)
+ABFIT_HD inline uint64_t param_boot_seed(uint64_t seed, uint64_t problem_id, uint64_t b)
+{
+    uint64_t h = mix64(seed ^ (6 * 0xd1342543de82ef95ull));
+    h = mix64(h ^ problem_id);
+    return mix64(h ^ b);
+}
+
 }  // namespace abfit

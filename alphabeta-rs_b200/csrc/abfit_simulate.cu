@@ -15,6 +15,7 @@
 #include <string>
 
 #include "abfit_internal.h"
+#include "abfit_psim.cuh"
 
 struct abfit_sim_tree {
     std::vector<int32_t> parent, gen;
@@ -29,7 +30,6 @@ namespace {
 
 constexpr int SIM_TILE = 256;                   // sites per block = threads per block
 constexpr int SIM_SMEM_MAX_NODES = 400;         // 100 KB of node states per block; larger forests use global scratch
-constexpr uint64_t SIM_STREAM = 4;              // generator stream (1: start simplices, 2: vary vertices, 3: resamples)
 
 struct SimNode {
     double c[6];                   // (c0, c1) per parent state
@@ -38,15 +38,6 @@ struct SimNode {
     int32_t parent_pos;            // position of the parent in the walk, -1 for a root
     int32_t out_row;               // output row, -1 when not sampled
 };
-
-ABFIT_HD inline double sim_u01(uint64_t key, uint64_t site) { return (double)(mix64(key ^ site) >> 11) * (1.0 / 9007199254740992.0); }
-
-uint64_t sim_key(uint64_t seed, int node, uint64_t which)
-{
-    uint64_t h = mix64(seed ^ (SIM_STREAM * 0xd1342543de82ef95ull));
-    h = mix64(h ^ (uint64_t)node);
-    return mix64(h ^ which);
-}
 
 __global__ void __launch_bounds__(SIM_TILE) k_simulate(const SimNode *__restrict__ nodes, int n_nodes, int64_t first_site,
                                                         int64_t L, double missing_rate, int with_missing,
@@ -214,6 +205,30 @@ int make_tree(int32_t n, const int32_t *parent, const int32_t *gen, const uint8_
 }
 
 }  // namespace
+
+void sim_walk(const abfit_sim_tree *t, std::vector<int32_t> &parent_pos, std::vector<int32_t> &node_id,
+              std::vector<int32_t> &row_pos)
+{
+    const int n = (int)t->parent.size();
+    std::vector<int32_t> pos(n);
+    for (int i = 0; i < n; ++i) pos[t->order[i]] = i;
+    parent_pos.resize(n);
+    node_id.assign(t->order.begin(), t->order.end());
+    row_pos.clear();
+    for (int i = 0; i < n; ++i) parent_pos[i] = t->parent[t->order[i]] < 0 ? -1 : pos[t->parent[t->order[i]]];
+    for (int v = 0; v < n; ++v)
+        if (t->sampled[v]) row_pos.push_back(pos[v]);
+}
+
+int sim_thresholds_walk(const abfit_sim_tree *t, const abfit_sim_params *params, double *out)
+{
+    if (int rc = check_params(params)) return rc;
+    const int n = (int)t->parent.size();
+    std::vector<double> thr((size_t)n * 6);
+    thresholds(*t, *params, thr.data());
+    for (int i = 0; i < n; ++i) std::memcpy(out + (size_t)i * 6, &thr[(size_t)t->order[i] * 6], 6 * sizeof(double));
+    return 0;
+}
 
 int run_simulate(cudaStream_t st, int n_sms, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
                  int64_t L, uint8_t *status, double *posterior_max, double *meth_lvl, bool device_out, float *kernel_ms)

@@ -507,6 +507,45 @@ int abfit_simulate(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_p
 int abfit_simulate_device(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_sim_params *params, int64_t first_site,
                           int64_t L, uint8_t *d_status, double *d_posterior_max, double *d_meth_lvl, float *kernel_ms);
 
+/* ---- parametric bootstrap and goodness of fit --------------------------------------------------
+ * Does ABneutral describe a window at all?  The LSE of the best fit is unscaled; abfit_param_boot_batch calibrates it:
+ * every replicate is a data set simulated from the window's FITTED model with the observed design, refitted, and the
+ * observed LSE is compared with the replicates' LSEs.  Windows share one forest `tree`: every problem's pedigree rows
+ * must be abfit_sim_tree_pairs(tree)'s (t0, t1, t2), in that order (else ABFIT_ERR_ARG before any launch).
+ *  Replicate b of window p, key k = problem_ids[p] (or first_problem_id + p): abfit_simulate(tree, {alpha = theta0,
+ *  beta = theta1, weight = theta2, p0uu = probs[p].p0uu, missing rates missing[p][s] per sample, seed =
+ *  abfit_gen_param_boot_seeds(seed, k)[b]}, first_site 0, L = n_sites[p]); with all rates of a window equal to m the
+ *  sites are abfit_simulate's with missing_rate = m.  D*[b][row] = diff / (2.0 * cnt) + theta3 from the exact integer
+ *  sums of the row's pair over the valid sites (posterior_max >= thr), which never leave the GPU as site arrays; adding
+ *  theta3 (the fit's intercept, the measurement error the simulator leaves out) is the only rounding besides the
+ *  division.  A replicate with a cnt = 0 row is not fitted (NaN row, ABFIT_FIT_NAN, counted in nan_reps_out).  Every
+ *  other replicate is refitted exactly like abfit_site_boot_batch's: from the simplex [best, vary x 4], vary =
+ *  abfit_gen_vary_vertices(seed, k, n_boot, best[p].theta), with the problem's p0uu, eqp and eqp_weight.  The refits
+ *  therefore start from the fitted model, not from fresh random starts: gof_p measures the fit as the replicates'
+ *  optimiser finds it near the truth, which favours the replicates slightly (smaller LSEs) and makes the test
+ *  conservative in that direction.
+ *  lse_star_out [n_probs][n_boot]  the penalty-free LSE of every refit against its D* (abfit_cost_batch's lse_out of
+ *                the refit theta on that column; NaN for unfitted replicates)
+ *  gof_p_out [n_probs]  (1 + #{b : lse_star >= best[p].lse}) / (1 + replicates whose status is not ABFIT_FIT_NAN)
+ *  window_status_out [n_probs]  0, or 1: theta0, theta1, theta2 or p0uu outside [0, 1], or a theta not finite (fitted
+ *                rates may be negative, the model cannot be simulated then); such a window gets no launch, NaN rows,
+ *                fits, analysis, D*, lse_star and p, and nan_reps 0.  The other windows are unchanged by it.
+ *  n_sites [n_probs] sites per window, 1 .. 2^31 - 1;  missing [n_probs][S] per-sample missing rates in [0, 1] or NULL
+ *                (no missing sites; tools pass 1 - nvalid / L of the observed window)
+ *  rows_out [n_probs][n_boot][7] (required), fits_out, analysis_out, dstar_out, nan_reps_out as abfit_site_boot_batch's
+ *                (each may be NULL), as are lse_star_out, gof_p_out and window_status_out.
+ * No site array is an input, so there is no _device twin.  Refused before any launch with ABFIT_ERR_TOO_LARGE: more than
+ * 200 sampled nodes, n_boot > 65535, a window of 2^31 sites or more, a forest whose nodes, samples and rows need more
+ * shared memory than a block has (8 + 256 bytes per node, 104 per sample, 4 per row), and outputs plus scratch that do
+ * not fit in free device memory. */
+void abfit_gen_param_boot_seeds(uint64_t seed, uint64_t problem_key, int32_t n_boot, uint64_t *seeds_out /* [n_boot] */);
+int abfit_param_boot_batch(abfit_ctx *ctx, const abfit_sim_tree *tree, const abfit_problem *probs, int32_t n_probs,
+                           const int64_t *n_sites, const double *missing, double thr, const abfit_fit *best, int32_t n_boot,
+                           uint64_t seed, uint64_t first_problem_id, const uint64_t *problem_ids, int32_t max_iters,
+                           double sd_tol, uint32_t flags, double *rows_out, abfit_fit *fits_out, double *analysis_out,
+                           double *dstar_out, double *lse_star_out, double *gof_p_out, int32_t *window_status_out,
+                           int32_t *nan_reps_out);
+
 /* ---- the reference's pictures (host; src/plot.rs) ------------------------------------
  * 1280 x 960 PNG files with the reference's series, colours, axis ranges and captions (not its pixels: own
  * rasteriser and bitmap font, see csrc/abfit_plot.cu).

@@ -17,6 +17,12 @@ use std::os::raw::{c_char, c_int};
 pub struct abfit_ctx {
     _p: [u8; 0],
 }
+
+/// a pedigree forest to simulate on (include/abfit.h, abfit_sim_tree_build)
+#[repr(C)]
+pub struct abfit_sim_tree {
+    _p: [u8; 0],
+}
 #[repr(C)]
 pub struct abfit_batch {
     _p: [u8; 0],
@@ -140,6 +146,17 @@ extern "C" {
         block_sites: i64, best: *const abfit_fit, n_boot: i32, seed: u64, first_problem_id: u64, problem_ids: *const u64,
         max_iters: i32, sd_tol: f64, flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit, analysis_out: *mut f64,
         dstar_out: *mut f64, nan_reps_out: *mut i32,
+    ) -> c_int;
+    /// parametric bootstrap: the simulator seeds [n_boot] of a window's replicates (generator stream 6)
+    pub fn abfit_gen_param_boot_seeds(seed: u64, problem_key: u64, n_boot: i32, seeds_out: *mut u64);
+    /// parametric bootstrap and goodness of fit of fitted windows on one pedigree forest: replicates simulated from the
+    /// fitted model and counted to exact D* on the GPU, refitted like the site bootstrap; gof_p ranks the observed LSE
+    pub fn abfit_param_boot_batch(
+        ctx: *mut abfit_ctx, tree: *const abfit_sim_tree, probs: *const abfit_problem, n_probs: i32, n_sites: *const i64,
+        missing: *const f64, thr: f64, best: *const abfit_fit, n_boot: i32, seed: u64, first_problem_id: u64,
+        problem_ids: *const u64, max_iters: i32, sd_tol: f64, flags: u32, rows_out: *mut f64, fits_out: *mut abfit_fit,
+        analysis_out: *mut f64, dstar_out: *mut f64, lse_star_out: *mut f64, gof_p_out: *mut f64,
+        window_status_out: *mut i32, nan_reps_out: *mut i32,
     ) -> c_int;
     /// one BED line -> (chromosome, 0-based start, end): 0 parsed, 1 not a region (empty, '#', track, browser), < 0 malformed
     pub fn abfit_parse_region_line(line: *const c_char, chrom_out: *mut i32, start0_out: *mut i64, end_out: *mut i64) -> c_int;
